@@ -558,6 +558,14 @@ def setup_model(args, n_max, local, sd=None):
     return model, engine, net, sd
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each array as ``out_dir/<name>.npy``: the inputs are seeded, so two builds can be compared array by array."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64) and a.nbytes <= 64 << 20, (name, a.dtype, a.nbytes)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_config2(args):
     import torch
     d = Dist()
@@ -569,6 +577,13 @@ def run_config2(args):
     model, engine, net, sd = setup_model(args, n_max, d.local)
     gather = ScoreGather(d, scan_rows, BATCH * PTS_PER_SCAN, every=args.gather_every)
     pending = []
+    last = [None]      # handle of the most recent finished step
+
+    def finish_one():
+        kk, p = pending.pop(0)
+        p.result()
+        gather.publish(p.device_scores, kk)
+        last[0] = p
 
     def step(inputs):
         def fn(k):
@@ -576,16 +591,12 @@ def run_config2(args):
             # are waited for inside the timed region, then the scan rows go to every rank on the comm stream
             pending.append((k, model.forward_async(inputs[k % len(inputs)])))
             if len(pending) >= model.lanes:
-                kk, p = pending.pop(0)
-                p.result()
-                gather.publish(p.device_scores, kk)
+                finish_one()
         return fn
 
     def drain():
         while pending:
-            kk, p = pending.pop(0)
-            p.result()
-            gather.publish(p.device_scores, kk)
+            finish_one()
         gather.flush()
 
     def measure(inputs, steps):
@@ -600,6 +611,8 @@ def run_config2(args):
     sampler = ClockSampler(d.local, enabled=d.rank == 0)
     sampler.start()
     ms_dev = measure(dev, args.steps)       # inputs resident in HBM
+    # the last timed step's scores, copied before the next window reuses the lane's buffer
+    outputs = {"scores": last[0].device_scores.cpu().numpy()} if args.dump_outputs and d.rank == 0 else None
     ms_host = measure(host, args.steps)     # public host-side API: pinned H2D of step k+1 overlaps the kernels of step k
     clocks = sampler.stop()
     engine.status()
@@ -673,6 +686,8 @@ def run_config2(args):
                            "flops_per_step": int(sum(a.get("flops", 0) for a in acc.values()))}
         if d.world == 1 and not args.no_cpu_baseline:
             result["cpu_baseline"] = cpu_baseline(batches[0], sd)
+        if outputs:
+            dump_outputs(args.dump_outputs, outputs)
     d.close()
     if d.rank == 0:
         print(json.dumps(result))
@@ -857,7 +872,11 @@ def main():
                     help="multi-GPU: steps whose scan-row scores (and metric partials) share one NCCL all-gather")
     ap.add_argument("--lanes", type=int, default=3, help="engine contexts/streams forward_async alternates between")
     ap.add_argument("--widths", default="1,2,4,8", help="config 5: PLANES multipliers of the sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="config 2: write the fp32 scores of the last device-resident timed step to DIR/scores.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs is implemented for --config 2 of --impl ours")
     args.steps_given = args.steps is not None
     if args.steps is None:
         args.steps = 20

@@ -1,57 +1,10 @@
-"""The MinkowskiEngine-shaped layer API (sps_b200.minkowski).
-
-CPU part: when the reference checkout is present (this container only -- never on the GPU box), its
-own ``minkunet.py`` / ``customminkunet.py`` are imported UNMODIFIED against the shim and must
-produce exactly the checkpoint layout the engine expects.  GPU part: a MinkUNet14 built from shim
-layers (graph restated here from minkunet.py:52-219) runs layer by layer and must agree with the
-fused forward and the oracle."""
-import importlib.util
-import os
-import sys
-
+"""The MinkowskiEngine-shaped layer API (sps_b200.minkowski): a MinkUNet14 built from shim layers
+(graph restated here from minkunet.py:52-219) runs layer by layer and must agree with the fused
+forward and the oracle; the reference's prune call sequence runs through the shim as written."""
 import numpy as np
 import pytest
 import torch
 import torch.nn as nn
-
-REF = "/root/reference/src/sps/models/MinkowskiEngine"
-
-
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not available (GPU box)")
-def test_reference_minkunet_imports_against_the_shim_and_matches_checkpoint_layout():
-    from sps_b200 import minkowski
-    from sps_b200.models import CustomMinkUNet
-    saved = {k: sys.modules.get(k) for k in list(sys.modules) if k.startswith("MinkowskiEngine") or k.startswith("sps.")}
-    minkowski.install()
-    try:
-        import types
-        for name in ("sps", "sps.models", "sps.models.MinkowskiEngine"):
-            sys.modules.setdefault(name, types.ModuleType(name))
-        mods = {}
-        for fname in ("resnet", "minkunet", "customminkunet"):
-            full = f"sps.models.MinkowskiEngine.{fname}"
-            spec = importlib.util.spec_from_file_location(full, os.path.join(REF, fname + ".py"))
-            mod = importlib.util.module_from_spec(spec)
-            mod.__package__ = "sps.models.MinkowskiEngine"
-            sys.modules[full] = mod
-            spec.loader.exec_module(mod)
-            mods[fname] = mod
-        torch.manual_seed(0)
-        ref_net = mods["customminkunet"].CustomMinkUNet(in_channels=1, out_channels=1, D=4)
-        mine = CustomMinkUNet()
-        a, b = ref_net.state_dict(), mine.state_dict()
-        assert set(a) == set(b)
-        for k in a:
-            assert tuple(a[k].shape) == tuple(b[k].shape), k
-        # weight_initialization of the reference (resnet.py:87-94) ran through the shim's kaiming_normal_
-        w = a["block5.0.conv1.kernel"]
-        assert abs(w.std().item() - np.sqrt(2.0 / (81 * 64))) < 2e-3
-    finally:
-        for k in [k for k in sys.modules if k.startswith("MinkowskiEngine") or k.startswith("sps.")]:
-            del sys.modules[k]
-        for k, v in saved.items():
-            if v is not None:
-                sys.modules[k] = v
 
 
 class ShimUNet(nn.Module):
