@@ -294,6 +294,39 @@ int sps_submap_ball_query(const sps_ballmap* bm, const float* d_scan_xyz, int64_
                           int32_t* d_offsets, int32_t* d_out_idx, int64_t out_capacity, int32_t* d_total,
                           void* d_scratch, size_t scratch_bytes, void* stream);
 
+/* A whole evaluation batch from its scans: BLTDataset.__getitem__ per scan (blt_dataset.py:209-243, no augmentation)
+ * + collate_fn (blt_dataset.py:173-182).  d_scans fp32 [n_total, ld >= 4] = x, y, z, label of `batch` scans already in
+ * the map frame, concatenated; h_offsets (HOST) int64 [batch + 1]: scan b = rows h_offsets[b] .. h_offsets[b+1], with
+ * h_offsets[0] == 0, non-decreasing, n_total = h_offsets[batch]; batch in 1..255 (the batch index is the voxel key's
+ * b field).  d_rows fp32 [row_capacity, 6] = (b, x, y, z, t, label) in collate order: for b = 0..batch-1 the scan
+ * rows of b (t = 1, their label), then b's submap rows map[idx] (t = 0, label 1), idx exactly what
+ * sps_submap_ball_query returns for that scan alone (same order, duplicates kept).  d_row_offsets int32 [batch + 1]:
+ * scan b's rows start at d_row_offsets[b]; *d_n_rows = number of rows.  When that exceeds row_capacity nothing is
+ * written past the capacity, and *d_n_rows and d_row_offsets still hold the true values (the caller compares after
+ * its synchronisation).  d_scratch: sps_radius_batch_scratch_bytes(n_total, batch) bytes, 256-byte aligned.
+ * No host synchronisation.  SPS_ERR_BAD_ARG: a null pointer, ld < 4, batch outside 1..255, offsets not starting at 0
+ * or decreasing, misaligned scratch; SPS_ERR_CAPACITY: scratch too small. */
+size_t sps_radius_batch_scratch_bytes(int64_t n_scan_total, int batch);
+int sps_radius_batch(const sps_ballmap* bm, const float* d_scans, int64_t ld, const int64_t* h_offsets, int batch,
+                     float* d_rows, int64_t row_capacity, int32_t* d_row_offsets, int32_t* d_n_rows, void* d_scratch,
+                     size_t scratch_bytes, void* stream);
+/* scripts/predict.py:70-83 over such a batch in one call: sps_radius_batch -> SPSModel.forward on the rows
+ * (models.py:20-30; the row count stays on the device, as in sps_infer_scan) -> SPSNet.predict_step's per-scan metric
+ * partials (models.py:84-104).  d_scan_scores fp32 [n_total]: the scores of the scan rows, in input order;
+ * d_counts int64 [batch][4] and d_sums double [batch][5]: per scan, laid out as in sps_confusion_counts (threshold eps).
+ * The rows are written to d_rows as by sps_radius_batch; the scores of all rows go to the context's own buffer.
+ * row_capacity sizes the forward's launches and, like a row count, decides the shape sort of sps_ctx_set_pattern_sort
+ * mode 1: pick it on the same side of 400 000 as the row count for scores bit-identical to sps_forward on the rows.
+ * When the rows do not fit row_capacity, the forward runs on none of them, the scan scores are NaN, the partials zero,
+ * *d_n_rows holds the true count and the context's status word reports SPS_ERR_CAPACITY at the next sps_ctx_status.
+ * No host synchronisation.  Errors as sps_radius_batch, plus SPS_ERR_CAPACITY when row_capacity > the context's
+ * max_points. */
+int sps_predict_radius_batch(sps_ctx* ctx, const sps_net* net, const sps_ballmap* bm, const float* d_scans, int64_t ld,
+                             const int64_t* h_offsets, int batch, float* d_rows, int64_t row_capacity,
+                             int32_t* d_row_offsets, int32_t* d_n_rows, void* d_scratch, size_t scratch_bytes,
+                             float voxel_size, float eps, float* d_scan_scores, int64_t* d_counts, double* d_sums,
+                             void* stream);
+
 /* ---------------------------------------------------------------- arithmetic / processing order ---- */
 /* Which kernels serve the fused forward of a context (and, through sps_conv_args.backend, one sps_conv_fwd call):
  *   SPS_BACKEND_AUTO (0)  tcgen05 implicit GEMM on fp16 rows (fp16 operands, fp32 accumulate and epilogue); the

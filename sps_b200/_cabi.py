@@ -33,6 +33,7 @@ SYMBOLS = [
     "sps_confusion_counts", "sps_voxel_mean", "sps_voxel_sum", "sps_gather_rows", "sps_affine_relu",
     "sps_pointcloud2_unpack", "sps_transform_points", "sps_pointcloud2_pack_scratch_bytes", "sps_pointcloud2_pack",
     "sps_ballmap_bytes", "sps_ballmap_build", "sps_ballmap_destroy", "sps_ball_query_scratch_bytes", "sps_submap_ball_query",
+    "sps_radius_batch_scratch_bytes", "sps_radius_batch", "sps_predict_radius_batch",
 ]
 
 
@@ -135,6 +136,10 @@ def load() -> C.CDLL:
         "sps_ballmap_destroy": (i32, [vp]),
         "sps_ball_query_scratch_bytes": (sz, [i64]),
         "sps_submap_ball_query": (i32, [vp, vp, i64, vp, vp, i64, vp, vp, sz, vp]),
+        "sps_radius_batch_scratch_bytes": (sz, [i64, i32]),
+        "sps_radius_batch": (i32, [vp, vp, i64, vp, i32, vp, i64, vp, vp, vp, sz, vp]),
+        "sps_predict_radius_batch": (i32, [vp, vp, vp, vp, i64, vp, i32, vp, i64, vp, vp, vp, sz, f32, f32, vp, vp, vp,
+                                           vp]),
         "sps_profile_enable": (i32, [vp, i32]),
         "sps_profile_read": (i32, [vp, vp, vp, i32, C.POINTER(i32)]),
         "sps_ctx_pair_count": (i32, [vp, i32, i32, C.POINTER(i64), vp]),

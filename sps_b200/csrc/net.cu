@@ -254,9 +254,11 @@ extern "C" int sps_net_finalize(sps_net* net, void* d_weights, size_t bytes, voi
 
 namespace sps {
 
-// SparseTensor.slice(tensor_field) + sigmoid (src/sps/models/models.py:28-29)
+// SparseTensor.slice(tensor_field) + sigmoid (src/sps/models/models.py:28-29); n_ptr (optional): the device row count,
+// rows at or past it are left untouched
 __global__ void k_devox_sigmoid(const float* __restrict__ logits, const int32_t* __restrict__ inv, int64_t n,
-                                float* __restrict__ scores, int apply_sigmoid) {
+                                float* __restrict__ scores, int apply_sigmoid, const int32_t* __restrict__ n_ptr) {
+  if (n_ptr && *n_ptr < n) n = *n_ptr;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const int v = __ldg(inv + i);
     float s = nanf("");
@@ -413,12 +415,13 @@ extern "C" int sps_unet_forward(sps_ctx* ctx, const sps_net* net, const float* d
   return unet_forward(ctx, net, d_feat0, d_logits, (cudaStream_t)stream);
 }
 
-static int devox(const float* d_logits, const int32_t* d_inv, int64_t n, float* d_scores, int apply_sigmoid, void* stream) {
+static int devox(const float* d_logits, const int32_t* d_inv, int64_t n, float* d_scores, int apply_sigmoid, void* stream,
+                 const int32_t* d_n = nullptr) {
   if (!d_logits || !d_inv || !d_scores || n < 0) return SPS_ERR_BAD_ARG;
   if (n == 0) return SPS_OK;
   int64_t g = (n + 255) / 256;
   if (g > 148 * 16) g = 148 * 16;
-  k_devox_sigmoid<<<(int)g, 256, 0, (cudaStream_t)stream>>>(d_logits, d_inv, n, d_scores, apply_sigmoid);
+  k_devox_sigmoid<<<(int)g, 256, 0, (cudaStream_t)stream>>>(d_logits, d_inv, n, d_scores, apply_sigmoid, d_n);
   SPS_CUDA_CHECK(cudaGetLastError());
   return SPS_OK;
 }
@@ -474,7 +477,7 @@ static int forward_feat_impl(sps_ctx* ctx, const sps_net* net, const float* d_po
   if (rc != SPS_OK) return rc;
   rc = unet_forward(ctx, net, ctx->buf[sps_ctx::FEAT0], ctx->buf[sps_ctx::LOGITS], st, /*conv0_done=*/true);
   if (rc != SPS_OK) return rc;
-  rc = devox(ctx->buf[sps_ctx::LOGITS], ctx->inv, n_scores, d_scores, net->apply_sigmoid, st);
+  rc = devox(ctx->buf[sps_ctx::LOGITS], ctx->inv, n_scores, d_scores, net->apply_sigmoid, st, d_n);
   if (rc != SPS_OK) return rc;
   prof_mark(ctx, "devox_sigmoid", st);
   ctx->forward_launches += 4 + 1;   // voxelise (4) and the devoxelisation; build_maps_impl / run_conv count their own

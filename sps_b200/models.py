@@ -10,6 +10,7 @@ computed inline.  Training (models.py:62-82,154-160) is out of scope (inference-
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 import os
 
@@ -18,7 +19,10 @@ import torch
 import torch.nn as nn
 
 from . import util
-from .engine import Engine, Net, norm_device
+from ._cabi import SPS_ERR_CAPACITY, SpsError, check
+from .datasets import MAX_BATCH, batch_parts
+from .engine import Engine, Net, _ptr, _stream, norm_device
+from .parallel import per_scan_metrics
 
 PLANES = (8, 16, 32, 64, 64, 32, 16, 8)   # customminkunet.py:11
 INIT_DIM = 8                              # customminkunet.py:12
@@ -145,6 +149,27 @@ class _Pending:
         return self._out
 
 
+class _PendingRadius:
+    """Handle of an in-flight ``SPSModel.predict_radius_async`` call."""
+
+    def __init__(self, event, out, engine, n_rows, retry):
+        self._event, self._out, self._engine, self._n_rows, self._retry = event, out, engine, n_rows, retry
+
+    def result(self, check: bool = True):
+        """Wait for the call and return ``(scan_scores, counts, sums)``.  ``check`` (default) also reads the engine's
+        sticky status word: a coordinate outside the voxel-key range raises here; rows that did not fit the lane's
+        context make the call run once more with contexts of the true row count."""
+        self._event.synchronize()
+        if check:
+            try:
+                self._engine.status()
+            except SpsError as e:
+                if e.code != SPS_ERR_CAPACITY:
+                    raise
+                return self._retry(int(self._n_rows[0])).result(check)
+        return self._out
+
+
 class SPSModel(nn.Module):
     def __init__(self, voxel_size: float, max_points: int = 0):
         super().__init__()
@@ -241,23 +266,8 @@ class SPSModel(nn.Module):
         if device.type != "cuda":
             raise RuntimeError("move the model to a CUDA device first: sps_b200 has no CPU path")
         n, ld = coordinates.shape
-        engine, net = self._prepare(n, device)
-        p = self._pipe
-        if p is None or p["cap"] < n or p["ld"] != ld:
-            cap = max(n, engine.max_points)
-            # two complete lanes (engine context + stream + staging buffers): consecutive calls alternate,
-            # so the hash/kernel-map phase of one call overlaps the convolution phase of the other
-            p = self._pipe = {"cap": cap, "ld": ld, "k": 0, "copy": torch.cuda.Stream(device=device),
-                              "engine": [engine] + [self._new_engine(engine.max_points, device) for _ in range(self.lanes - 1)],
-                              "stream": [torch.cuda.Stream(device=device) for _ in range(self.lanes)],
-                              "d_in": [torch.empty((cap, ld), dtype=torch.float32, device=device) for _ in range(self.lanes)],
-                              "d_out": [torch.empty(cap, dtype=torch.float32, device=device) for _ in range(self.lanes)],
-                              "h_out": [torch.empty(cap, dtype=torch.float32).pin_memory() for _ in range(self.lanes)],
-                              "busy": [None] * self.lanes, "graphs": [dict() for _ in range(self.lanes)]}
-        slot = p["k"] % self.lanes
-        p["k"] += 1
-        if p["busy"][slot] is not None:
-            p["busy"][slot].synchronize()          # the buffers of this lane are free again
+        p, net = self._lanes(n, ld, device)
+        slot = self._next_lane(p)
         lane_engine, compute = p["engine"][slot], p["stream"][slot]
         d_in, d_out, h_out = p["d_in"][slot][:n], p["d_out"][slot][:n], p["h_out"][slot][:n]
         compute.wait_stream(torch.cuda.current_stream(device))
@@ -282,6 +292,120 @@ class SPSModel(nn.Module):
         p["busy"][slot] = done
         engine = lane_engine
         return _Pending(done, h_out, engine, device_scores=d_out)
+
+    def _lanes(self, n, ld, device):
+        """The lanes of the pipelined entry points, (re)made for inputs of up to ``n`` rows of width ``ld`` (None: any
+        width; a new set of lanes then takes 5)."""
+        engine, net = self._prepare(n, device)
+        p = self._pipe
+        if p is None or p["cap"] < n or (ld is not None and p["ld"] != ld):
+            cap = max(n, engine.max_points)
+            ld = ld or 5
+            # two complete lanes (engine context + stream + staging buffers): consecutive calls alternate,
+            # so the hash/kernel-map phase of one call overlaps the convolution phase of the other
+            p = self._pipe = {"cap": cap, "ld": ld, "k": 0, "copy": torch.cuda.Stream(device=device),
+                              "engine": [engine] + [self._new_engine(engine.max_points, device) for _ in range(self.lanes - 1)],
+                              "stream": [torch.cuda.Stream(device=device) for _ in range(self.lanes)],
+                              "d_in": [torch.empty((cap, ld), dtype=torch.float32, device=device) for _ in range(self.lanes)],
+                              "d_out": [torch.empty(cap, dtype=torch.float32, device=device) for _ in range(self.lanes)],
+                              "h_out": [torch.empty(cap, dtype=torch.float32).pin_memory() for _ in range(self.lanes)],
+                              "busy": [None] * self.lanes, "graphs": [dict() for _ in range(self.lanes)],
+                              "radius": [dict() for _ in range(self.lanes)]}
+        return p, net
+
+    def _next_lane(self, p):
+        """The lane of the next call, once the call that used it before is done with its buffers."""
+        slot = p["k"] % self.lanes
+        p["k"] += 1
+        if p["busy"][slot] is not None:
+            p["busy"][slot].synchronize()          # the buffers of this lane are free again
+        return slot
+
+    def predict_radius_async(self, scans, submap, eps: float, offsets=None):
+        """``scripts/predict.py``'s loop body for a whole batch in one asynchronous library call: for every scan its
+        radius submap from ``submap`` (a :class:`sps_b200.datasets.RadiusSubmap` of the base map, radius =
+        VOXEL_SIZE), the collated rows (``RadiusSubmap.make_batch``), ``forward`` on them and ``predict_step``'s metric
+        partials per scan (threshold ``eps``).  ``scans``: a list of per-scan fp32 ``[n_b, >=4]`` tensors (x, y, z,
+        label in the map frame) or one ``[sum n_b, >=4]`` tensor plus ``offsets`` (``B + 1`` ints).
+
+        Returns a handle whose ``result()`` gives ``(scan_scores [sum n_b], counts int64 [B, 4], sums float64 [B, 5])``
+        (layouts of ``parallel.device_partials``; ``parallel.per_scan_metrics`` turns them into predict.py's values).
+        Host scans go to the device on a copy stream into the staging buffer of one of the model's lanes (the copies of
+        call k+1 overlap the kernels of call k) and the results come back to pinned host memory; device scans are read
+        in place and the results stay on the device.  Either way the buffers belong to the lane: the call ``lanes``
+        calls later reuses them.  The row capacity is the lane context's size; rows that do not fit are never scored:
+        ``result()`` then grows the contexts to the true row count and runs the batch once more (the only extra host
+        synchronisation, on that path only)."""
+        if self.training:
+            raise RuntimeError("sps_b200 is inference-only (call .eval()); training is out of scope")
+        parts, offs, ld = batch_parts(scans, offsets)
+        return self._predict_radius(parts, offs, ld, submap, float(eps), 6 * offs[-1])
+
+    def _predict_radius(self, parts, offs, ld, submap, eps, rows_guess):
+        device = next(self.MinkUNet.parameters()).device
+        if device.type != "cuda":
+            raise RuntimeError("move the model to a CUDA device first: sps_b200 has no CPU path")
+        if submap.map_xyz.device != device:
+            raise RuntimeError("the submap's base map must live on the model's device")
+        n, batch = offs[-1], len(offs) - 1
+        p, net = self._lanes(max(rows_guess, 1), None, device)
+        slot = self._next_lane(p)
+        lane_engine, compute = p["engine"][slot], p["stream"][slot]
+        cap = lane_engine.max_points
+        on_device = all(t.is_cuda for t, _ in parts)
+        buf = p["radius"][slot]
+        lib = lane_engine.lib
+
+        def grow(name, shape, dtype, pinned=False):
+            t = buf.get(name)
+            if t is None or t.shape[0] < shape[0]:
+                t = torch.empty(shape, dtype=dtype, device="cpu" if pinned else device)
+                buf[name] = t.pin_memory() if pinned else t
+            return buf[name]
+
+        nbytes = lib.sps_radius_batch_scratch_bytes(n, batch)
+        rows = grow("rows", (cap, 6), torch.float32)
+        scratch = grow("scratch", (nbytes,), torch.uint8)    # the caching allocator hands out 512-byte aligned blocks
+        row_offsets = grow("row_offsets", (MAX_BATCH + 1,), torch.int32)
+        n_rows = grow("n_rows", (1,), torch.int32)
+        scores = grow("scores", (max(n, 1),), torch.float32)
+        counts = grow("counts", (MAX_BATCH, 4), torch.int64)
+        sums = grow("sums", (MAX_BATCH, 5), torch.float64)
+        compute.wait_stream(torch.cuda.current_stream(device))
+        if len(parts) == 1 and on_device and parts[0][0].device == device:
+            src = parts[0][0]
+        else:
+            src = grow(("scans", ld), (max(n, 1), ld), torch.float32)
+            copy = compute if on_device else p["copy"]
+            with torch.cuda.stream(copy):
+                for t, start in parts:
+                    src[start:start + t.shape[0]].copy_(t, non_blocking=True)
+                ready = torch.cuda.Event()
+                ready.record(copy)
+            compute.wait_event(ready)
+        buf["keep"] = (parts, src)                          # alive until the lane's next call
+        h_off = (C.c_int64 * (batch + 1))(*offs)
+        with torch.cuda.device(device), torch.cuda.stream(compute):
+            check(lib.sps_predict_radius_batch(lane_engine.handle, net.handle, submap.handle, _ptr(src), ld, h_off, batch,
+                                               _ptr(rows), cap, _ptr(row_offsets), _ptr(n_rows), _ptr(scratch), nbytes,
+                                               self.voxel_size, eps, _ptr(scores), _ptr(counts), _ptr(sums),
+                                               _stream(device)), "sps_predict_radius_batch")
+            out = (scores[:n], counts[:batch], sums[:batch])
+            if not on_device:
+                h = (grow("h_scores", (max(n, 1),), torch.float32, True), grow("h_counts", (MAX_BATCH, 4), torch.int64, True),
+                     grow("h_sums", (MAX_BATCH, 5), torch.float64, True))
+                out = (h[0][:n], h[1][:batch], h[2][:batch])
+                for dst, s in zip(out, (scores[:n], counts[:batch], sums[:batch])):
+                    dst.copy_(s, non_blocking=True)
+            h_rows = grow("h_n_rows", (1,), torch.int32, True)
+            h_rows.copy_(n_rows, non_blocking=True)
+            done = torch.cuda.Event()
+            done.record(compute)
+        p["busy"][slot] = done
+
+        def retry(true_rows):
+            return self._predict_radius(parts, offs, ld, submap, eps, true_rows)
+        return _PendingRadius(done, out, lane_engine, h_rows, retry)
 
     def _lane_forward(self, p, slot, lane_engine, net, src, d_out, compute):
         """One forward on a lane's stream (current), eagerly or as a CUDA-graph replay.  Every size that only exists on
@@ -421,6 +545,22 @@ class SPSNet(nn.Module):
         self.recall.append(recall)
         self.F1.append(f1)
         return scores
+
+    @torch.no_grad()
+    def predict_scans(self, scans, submap, offsets=None):
+        """``predict_step`` for a batch of raw scans (``SPSModel.predict_radius_async``: radius submaps, collation,
+        forward and metric partials in the library): appends each scan's Loss / R2 / dIoU / Precision / Recall / F1 to
+        the lists ``predict_step`` fills -- the values predict.py gets with ``batch_size=1`` -- and returns the scan
+        rows' scores.  Scans without points add nothing."""
+        scan_scores, counts, sums = self.model.predict_radius_async(scans, submap, self.epsilon, offsets=offsets).result()
+        m = per_scan_metrics(counts, sums)
+        self.predict_loss += m["Loss"]
+        self.predict_r2 += m["R2"]
+        self.dIoU += m["dIoU"]
+        self.precision += m["Precision"]
+        self.recall += m["Recall"]
+        self.F1 += m["F1"]
+        return scan_scores
 
     def summary(self):
         """scripts/predict.py:70-83: mean over per-batch values (not pooled counts)."""

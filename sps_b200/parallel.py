@@ -77,9 +77,9 @@ def gather_partials(counts: torch.Tensor, sums: torch.Tensor, n_items: int):
     return oc, os_
 
 
-def metrics_from_partials(counts: torch.Tensor, sums: torch.Tensor) -> dict:
-    """scripts/predict.py:70-83 semantics: every metric is the MEAN over per-scan values (not pooled
-    counts); per-scan formulas from util.py:285-299 and models.py:91-92."""
+def per_scan_metrics(counts: torch.Tensor, sums: torch.Tensor) -> dict:
+    """The values ``SPSNet.predict_step`` appends for each scan (models.py:84-104, util.py:285-299), from its partials:
+    {metric: [value per scan]}; scans without points are skipped."""
     out = {"Loss": [], "R2": [], "dIoU": [], "Precision": [], "Recall": [], "F1": []}
     for (tp, tn, fp, fn), (n, sse, sl, sll, _ss) in zip(counts.tolist(), sums.tolist()):
         if n == 0:
@@ -95,7 +95,13 @@ def metrics_from_partials(counts: torch.Tensor, sums: torch.Tensor) -> dict:
         out["Precision"].append(precision)
         out["Recall"].append(recall)
         out["F1"].append(f1)
-    return {k: float(np.mean(v)) for k, v in out.items() if len(v)}
+    return out
+
+
+def metrics_from_partials(counts: torch.Tensor, sums: torch.Tensor) -> dict:
+    """scripts/predict.py:70-83 semantics: every metric is the MEAN over per-scan values (not pooled
+    counts); per-scan formulas from util.py:285-299 and models.py:91-92."""
+    return {k: float(np.mean(v)) for k, v in per_scan_metrics(counts, sums).items() if len(v)}
 
 
 def device_partials(scores: torch.Tensor, rows: torch.Tensor, eps: float):
