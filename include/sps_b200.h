@@ -69,15 +69,15 @@ typedef struct sps_level_view {
   const int32_t* parent;    /* [count] parent*8 + child-offset index into level+1 (NULL at 4)*/
   const int32_t* child;     /* [8][ld] child table of the level BELOW (NULL at level 0)     */
   int64_t ld;               /* leading dimension (in voxels) of nbr3/nbr5/child             */
-  /* Processing order of the 3x3x3x3 convolutions after a fused forward that shape-sorted this level (levels 0-3 of
-   * inputs >= 400 000 rows, or sps_ctx_set_pattern_sort(ctx, 2)); all NULL otherwise.  These are what
+  /* Processing order of the 3x3x3x3 convolutions after a fused forward that shape-sorted the levels (inputs of
+   * >= 400 000 rows, or sps_ctx_set_pattern_sort(ctx, 2)); all NULL otherwise.  These are what
    * sps_conv_args.perm / tile_mask / tile_slices take: a caller can run its own layers on the forward's maps. */
   const int32_t* perm;          /* [count] rows in neighbourhood-shape order                                  */
   const uint32_t* tile_mask;    /* [ceil(count/128)][4] present-offset masks of the tiles in that order       */
   const int32_t* tile_slices;   /* [tiles][SPS_TILE_SLICE_ENTRIES][128] kernel map gathered per tile          */
 } sps_level_view;
 /* Valid after sps_voxelize (+ sps_build_maps for the maps).  After a FUSED forward (sps_forward*, sps_infer_scan) on
- * an input large enough for the shape sort (>= 400 000 rows), the 3x3x3x3 tables of levels 0-3 hold only their PRESENT
+ * an input large enough for the shape sort (>= 400 000 rows), the 3x3x3x3 tables of all levels hold only their PRESENT
  * entries (absent ones are not rewritten to -1: every reader inside the library goes through the presence words):
  * the view then carries nbr3 == NULL for every level; call sps_build_maps to get the complete tables back
  * (sps_ctx_pair_count counts from the presence words and works in both states). */
@@ -341,7 +341,7 @@ int sps_predict_radius_batch(sps_ctx* ctx, const sps_net* net, const sps_ballmap
 #define SPS_BACKEND_TF32 2
 #define SPS_BACKEND_F16 3
 int sps_ctx_set_conv_backend(sps_ctx* ctx, int backend);
-/* The fused forward can visit the rows of the 3x3x3x3 convolutions (levels 0-3) in an order sorted by
+/* The fused forward can visit the rows of the 3x3x3x3 convolutions (all levels) in an order sorted by
  * neighbourhood shape: fewer kernel offsets per 128-row tile.  mode 0: never (physical row order); 1 (default): for
  * inputs of >= 400 000 rows (smaller ones are launch-bound); 2: always.  Results do not depend on it beyond the last
  * bit of a stored fp16 activation. */
@@ -366,8 +366,8 @@ int64_t sps_conv_kmajor_ld_f16s(int K, int cin, int cin2, int pack_flags, int ci
 int sps_conv_pack_kmajor_f16s(const float* w, int K, int cin, int cout, const float* w2, int cin2, int pack_flags, int cin_split,
                               void* out);
 /* 1 when the tensor-core kernel can stage its 64-channel weight slabs through TMA (cp.async.bulk.tensor): the driver's
- * cuTensorMapEncodeTiled was found (cudaGetDriverEntryPoint) and SPS_NO_TMA_B is not set in the environment; 0: every
- * weight stage goes through cp.async (same results). */
+ * cuTensorMapEncodeTiled was found (cudaGetDriverEntryPoint); 0: every weight stage goes through cp.async (same
+ * results). */
 int sps_tma_weights_available(void);
 /* Per-tile present-offset bitmasks of a kernel map (K <= 81) for the tensor-core path:
  * d_masks uint32 [ceil(n_out_max/128)][4]. */

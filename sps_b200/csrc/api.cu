@@ -56,7 +56,7 @@ static size_t carve(sps_ctx* c, void* base, int64_t max_points) {
     c->tmask3[L] = cv.take<uint32_t>((size_t)(ld / 128 + 1) * 4);
     c->ptmask[L] = cv.take<uint32_t>((size_t)(ld / 128 + 1) * 4);
     c->perm[L] = cv.take<int32_t>(N);
-    c->tslice[L] = (L <= 4) ? cv.take<int32_t>((size_t)(ld / 128 + 1) * SPS_TILE_SLICE_ENTRIES * 128) : nullptr;
+    c->tslice[L] = cv.take<int32_t>((size_t)(ld / 128 + 1) * SPS_TILE_SLICE_ENTRIES * 128);
     c->btab[L] = cv.take<Slot>(c->table_cap);
     c->bcells[L] = cv.take<int32_t>((size_t)N * 64);
     c->bocc[L] = cv.take<unsigned long long>(N);
@@ -167,10 +167,10 @@ extern "C" int sps_ctx_level(sps_ctx* ctx, int level, sps_level_view* v) {
   v->parent = ctx->parent[level];
   v->child = ctx->child[level];
   v->ld = ctx->ld;
-  const bool sorted = ctx->have_maps && ctx->have_perm && level >= ctx->first_sorted && level <= ctx->last_sorted;
+  const bool sorted = ctx->have_maps && ctx->have_perm;
   v->perm = sorted ? ctx->perm[level] : nullptr;
   v->tile_mask = sorted ? ctx->ptmask[level] : nullptr;
-  v->tile_slices = sorted && ctx->have_slices ? ctx->tslice[level] : nullptr;
+  v->tile_slices = sorted ? ctx->tslice[level] : nullptr;
   return SPS_OK;
 }
 

@@ -108,16 +108,13 @@ __host__ __device__ inline uint32_t hash_key(unsigned long long k) {
 // table capacity for n keys: smallest power of two >= max(1024, 1.5 n) -- load factor <= 0.67 if every key is distinct
 // (linear probing: ~2.5 probes per miss at that load), in practice 0.2-0.45 (2.3 input rows per voxel on the bench scans).
 // 2n would double the table: 134 MB instead of 67 MB for the 2.47 M-row batch, i.e. past the 126 MB L2.
-#ifndef SPS_TABLE_X2
-#define SPS_TABLE_X2 3      // capacity >= SPS_TABLE_X2 / 2 * n
-#endif
 __host__ __device__ inline uint32_t table_capacity(int64_t n) {
 #ifdef __CUDA_ARCH__
-  const unsigned long long need = ((unsigned long long)n * SPS_TABLE_X2 + 1) / 2;
+  const unsigned long long need = ((unsigned long long)n * 3 + 1) / 2;
   return need <= 1024ull ? 1024u : 1u << (64 - __clzll((long long)(need - 1)));
 #else
   uint32_t c = 1024;
-  while ((int64_t)c * 2 < n * SPS_TABLE_X2) c <<= 1;
+  while ((int64_t)c * 2 < n * 3) c <<= 1;
   return c;
 #endif
 }

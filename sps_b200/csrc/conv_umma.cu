@@ -30,15 +30,7 @@ namespace sps {
 // CTAs per SM, each with a 2-deep ring and one staged kernel-map slice (<= 113 KB of shared memory, <= 72 registers):
 // convolution family 1.79 -> 1.61 ms per forward (3-deep rings: 1.64) -- two independent gather streams fill the L1 data
 // pipe better than one deep ring, and the loader's bubble at a tile boundary hides behind the other CTA.
-#ifndef SPS_V6_S16
-#define SPS_V6_S16 2
-#endif
-#ifndef SPS_V6_S32
-#define SPS_V6_S32 2
-#endif
-#ifndef SPS_V6_S64
-#define SPS_V6_S64 2
-#endif
+constexpr int kV6CtasPerSm = 2;   // resident CTAs per SM for N <= 64 (the wide accumulators of the width sweep take a whole SM)
 constexpr int kV6ProducerWarps = 8;
 constexpr int kV6ProducerThreads = kV6ProducerWarps * 32;
 constexpr int kV6LoaderWarp = kV6ProducerWarps;
@@ -47,7 +39,7 @@ constexpr int kV6EpiWarp0 = kV6MmaWarp + 1;
 constexpr int kV6Threads = (kV6EpiWarp0 + 4) * 32;
 constexpr int kV6Entries = kMaxK + 1;                 // present offsets + the tile's own rows
 constexpr int kV6EntryBytes = kTileM * 4;
-// The index area (2 x 82 entries) holds as many tiles as fit: 2 for the 81-offset kernels, 8 for the 2x2x2 ones
+// The index area (82 entries) holds as many tiles as fit: 1 for the 81-offset kernels, 8 for the 2x2x2 ones
 // (9 entries per tile).  Tiles of the small kernels are one or two stages long, so the number of tiles in flight
 // -- not the stage ring -- bounds their memory-level parallelism.
 constexpr int kV6MaxTilesAhead = 8;
@@ -55,26 +47,20 @@ constexpr int kV6MaxTilesAhead = 8;
 // byte counts here: 167 936 bytes per CTA is the last size that still gets the 164 KB carve-out, i.e. 92 KB of L1.)
 constexpr int kV6KlistBytes = 256;
 
-#ifndef SPS_V6_PAD_KB
-#define SPS_V6_PAD_KB 0   // experiment: unused shared memory, shrinks the L1 side of the unified array
-#endif
 template <int NPAD>
 struct V6Cfg {
-  // SPS's own widths (N <= 64): 4 stages, two tiles of kernel-map slices staged.  Wide accumulators of the width sweep
-  // (N = 128 / 256, 16 / 32 KB of weights per stage): 4 / 3 stages and ONE staged slice -- a stage of such a layer keeps
-  // the tensor pipe busy for 256 / 512 cycles, the loader's bubble at a tile boundary is noise there.
-  static constexpr int S = NPAD == 256 ? 3 : NPAD == 128 ? 4 : NPAD == 64 ? SPS_V6_S64 : NPAD == 32 ? SPS_V6_S32 : SPS_V6_S16;
+  // SPS's own widths (N <= 64): 2 stages (above).  Wide accumulators of the width sweep (N = 128 / 256, 16 / 32 KB of
+  // weights per stage): 4 / 3 stages -- a stage of such a layer keeps the tensor pipe busy for 256 / 512 cycles, the
+  // loader's bubble at a tile boundary is noise there.  Every width stages one tile's kernel-map slice.
+  static constexpr int S = NPAD == 256 ? 3 : NPAD == 128 ? 4 : 2;
   static constexpr int kBStage = NPAD * 128;
   static constexpr int kTmemCols = 2 * NPAD < 32 ? 32 : 2 * NPAD;
-#ifndef SPS_V6_IDX_TILES
-#define SPS_V6_IDX_TILES 1
-#endif
-  static constexpr int kIdxEntries = NPAD >= 128 ? kV6Entries : SPS_V6_IDX_TILES * kV6Entries;
+  static constexpr int kIdxEntries = kV6Entries;
   static constexpr int kShift = NPAD < 64 ? 64 : NPAD;
   // A ring | B ring | row indices [kIdxEntries][128] | barriers | klists | nact [8] | shift | tmem slot
   static constexpr size_t smem = (size_t)S * (kAStageBytes + kBStage) + (size_t)kIdxEntries * kV6EntryBytes +
                                  8 * (2 * S + 2 * kV6MaxTilesAhead + 4) + kV6KlistBytes + 4 * kV6MaxTilesAhead +
-                                 kShift * 4 + 16 + SPS_V6_PAD_KB * 1024;
+                                 kShift * 4 + 16;
 };
 
 // 16-byte copy that writes zeros instead when `skip` is set (the ignore-src form: one predicate, no size select)
@@ -99,13 +85,8 @@ __device__ __forceinline__ void cp_async16_or_zero(uint32_t dst, const void* src
 }
 // The gathers of the A operand bypass L1 (cp.async.cg): measured alone the convolution family is 2 % SLOWER that way
 // (1.517 -> 1.553 ms, the 8- and 24-channel layers lose their L1 hits), but the three-lane step is 1.8 % FASTER (2.414 ->
-// 2.372 ms, reproduced twice): the gathered rows no longer evict the lines the other lanes' map kernels work on.
-#ifndef SPS_V6_A_CG
-#define SPS_V6_A_CG 1
-#endif
-#ifndef SPS_V6_B_CG
-#define SPS_V6_B_CG 0
-#endif
+// 2.372 ms, reproduced twice): the gathered rows no longer evict the lines the other lanes' map kernels work on.  The
+// weight copies keep L1 (cp.async.ca).
 __device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
 }
@@ -118,10 +99,7 @@ __device__ __forceinline__ void cp_async4(uint32_t dst, const void* src) {
 // 48 = 32 + 16 and 24 = 16 + 8 channels without a single padded column (1.5 / 0.75 / 0.375 stages per offset instead
 // of 2 / 1 / 0.5).
 template <int NPAD, int GPC, typename T, int GPC2 = 0>
-#ifndef SPS_V6_CTAS_PER_SM
-#define SPS_V6_CTAS_PER_SM 2   // resident CTAs per SM for N <= 64 (the wide accumulators of the width sweep take a whole SM)
-#endif
-__global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? SPS_V6_CTAS_PER_SM : 1) k_conv_umma6(const sps_conv_args a, const __grid_constant__ UmmaParams p) {
+__global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_conv_umma6(const sps_conv_args a, const __grid_constant__ UmmaParams p) {
   using Cfg = V6Cfg<NPAD>;
   constexpr int EB = sizeof(T);                         // bytes per stored activation
   constexpr bool kHalf = EB == 2;
@@ -346,7 +324,7 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? SPS_V6_CTAS_PER_SM : 
           for (int i = 0; i < 4; ++i) {
             const bool ok = okc && idx[i] >= 0;
             const uint32_t row = (uint32_t)(idx[i] < 0 ? 0 : idx[i]);
-            cp_async16_or_zero<SPS_V6_A_CG != 0>(dstA + a_off[i], base + (uint64_t)row * ld_b, !ok);
+            cp_async16_or_zero<true>(dstA + a_off[i], base + (uint64_t)row * ld_b, !ok);
           }
           if (stage_tma) {
             if (tid == 0) {   // thread 0 holds column 0 of the slab: wofs = byte offset of the slab in a weight row
@@ -356,7 +334,7 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? SPS_V6_CTAS_PER_SM : 
           } else if (b_lane) {
 #pragma unroll
             for (int i = 0; i < NB; ++i)
-              cp_async16_or_zero<SPS_V6_B_CG != 0>(sB_u + (uint32_t)s * kBStageBytes + b_off[i], wrow[i] + wofs, !(bok && wok[i]));
+              cp_async16_or_zero<false>(sB_u + (uint32_t)s * kBStageBytes + b_off[i], wrow[i] + wofs, !(bok && wok[i]));
           }
           cp_async_arrive(bar_full + 8 * s);          // fires when this thread's copies of the stage have landed
           more = advance();
@@ -595,7 +573,6 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn encode_tiled_fn() {
   static EncodeTiledFn fn = []() -> EncodeTiledFn {
-    if (getenv("SPS_NO_TMA_B")) return nullptr;     // A/B switch: weight stages through cp.async everywhere
     void* f = nullptr;
     cudaDriverEntryPointQueryResult q;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
@@ -627,7 +604,7 @@ static int launch_umma6(const sps_conv_args& a, const UmmaParams& p_in, cudaStre
   SPS_CUDA_CHECK(ensure_dynamic_smem(k_conv_umma6<NPAD, GPC, T, GPC2>, smem, &attr_done));
   int64_t tiles = (a.n_out_max + kTileM - 1) / kTileM;
   if (tiles < 1) tiles = 1;
-  const int per_sm = NPAD <= 64 ? SPS_V6_CTAS_PER_SM : 1;
+  const int per_sm = NPAD <= 64 ? kV6CtasPerSm : 1;
   const int grid = (int)(tiles < 148 * per_sm ? tiles : 148 * per_sm);
   k_conv_umma6<NPAD, GPC, T, GPC2><<<grid, kV6Threads, smem, st>>>(a, p);
   SPS_CUDA_CHECK(cudaGetLastError());

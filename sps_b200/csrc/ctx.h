@@ -11,9 +11,9 @@ struct sps_ctx {
   int64_t max_points = 0;
   int64_t ld = 0;            // leading dimension of the [K][ld] map tables (multiple of 32)
   int64_t n = 0;             // rows of the last voxelize call
-  bool have_l0 = false, have_maps = false, have_nbr5 = false, have_perm = false, have_slices = false;
-  bool dense_maps = true;    // false after a fused forward that stored only the present entries of the sorted levels' tables
-  int first_sorted = 0, last_sorted = -1;   // levels whose 3^4 convs may visit rows in pattern-sorted order
+  bool have_l0 = false, have_maps = false, have_nbr5 = false;
+  bool have_perm = false;    // the 3^4 convs of every level visit rows in pattern-sorted order (perm, ptmask, tslice are valid)
+  bool dense_maps = true;    // false after a fused forward that stored only the present entries of the sorted tables
 
   // ---- settings (sps_ctx_set_conv_backend / sps_ctx_set_pattern_sort) and per-forward state ----
   int backend = SPS_BACKEND_AUTO;
@@ -56,9 +56,9 @@ struct sps_ctx {
   uint32_t* vmask[SPS_NUM_LEVELS] = {};        // [L] [ld][4] per-voxel 27-bit presence words of the 3x3x3 neighbours in the three time planes (+ pad)
   int32_t* perm[SPS_NUM_LEVELS] = {};          // [L] rows of level L in neighbourhood-shape order (conv processing order)
   uint32_t* ptmask[SPS_NUM_LEVELS] = {};       // [L] tile masks of nbr3 in perm order
-  int32_t* tslice[SPS_NUM_LEVELS] = {};        // [L] [tiles][82][128] nbr3 gathered per tile in perm order (sorted levels)
-  // shape sort of levels 0..3 together (4 x max_points keys): ping-pong buffers, [4][256] digit histograms + 4 tile
-  // tickets, look-back status words [tiles][4][256]
+  int32_t* tslice[SPS_NUM_LEVELS] = {};        // [L] [tiles][82][128] nbr3 gathered per tile in perm order
+  // shape sort of all five levels together (5 x max_points keys): ping-pong buffers, [4][256] digit histograms of the four
+  // radix passes + 4 tile tickets, look-back status words [tiles][4][256]
   uint32_t* sort_keys[2] = {};
   int32_t* sort_vals[2] = {};
   uint32_t* sort_hist = nullptr;
@@ -88,12 +88,9 @@ struct Conv0Fused {
   float cfeat;
   const float* w; const float* shift; int round_out; float* out; int64_t out_ld;
 };
-// SPS_CAT_PAD=1 pads the row strides of the concat buffers to a power of two (24 -> 32, 48 -> 64, 96 -> 128 channels) so that a
-// gathered fp16 row never straddles a 128-byte line; measured neutral (block6.conv1 0.1685 ms either way), off by default.
-#ifndef SPS_CAT_PAD
-#define SPS_CAT_PAD 0
-#endif
-constexpr int kCatLd[4] = {16, SPS_CAT_PAD ? 32 : 24, SPS_CAT_PAD ? 64 : 48, SPS_CAT_PAD ? 128 : 96};   // CAT8, CAT7, CAT6, CAT5
+// Row strides of the concat buffers, unpadded: padding them to a power of two (so that a gathered fp16 row never straddles a
+// 128-byte line) measured neutral (block6.conv1 0.1685 ms either way).
+constexpr int kCatLd[4] = {16, 24, 48, 96};   // CAT8, CAT7, CAT6, CAT5
 constexpr int kBufWidth[sps_ctx::NBUF] = {16, 8, 8, kCatLd[1], 8, 16, kCatLd[2], 16, 32, kCatLd[3], 32, 64, 64, 64, 64, 32, 32,
                                           16, 16, 8, 1, 1};
 

@@ -20,9 +20,7 @@ constexpr uint32_t kInvalidSlot = 0xFFFFFFFFu;
 __global__ void k_set_i32(int32_t* p, int32_t v) { *p = v; }
 
 constexpr int kRankChunks = 4;    // chunks of kScanBlock rows a block of k_first_rank scans
-#ifndef SPS_SLICE_BATCH
-#define SPS_SLICE_BATCH 16
-#endif
+constexpr int kSliceBatch = 16;   // kernel-map entries a thread of k_tile_masks_perm reads before it stores them
 constexpr int kInsertBatch = 4;   // rows a thread of the level-0 insert kernel keeps in flight
 
 // First kernel of a level: empties the open-addressing table for `n` keys and, for a strided level, presets the
@@ -253,12 +251,16 @@ k_up_order(const UpOrderArgs A) {
 // 256-byte block instead of one random 32-byte sector of a per-voxel hash table.
 // The tables of ALL levels are built by the same three launches (blockIdx.y = level): the coarse levels hold a few
 // thousand voxels each and were pure launch latency as separate kernels.
+// Levels 0..2 build no block hash of their own: the 4x4x4 blocks of level L are the voxels of level L + 2, and the stride
+// chain's hash of those voxels answers "block key -> block row".  That hash was built from, and sized for, the rows of
+// level L + 1.
+__host__ __device__ constexpr bool blocks_are_voxels(int L) { return L + 2 < SPS_NUM_LEVELS; }
+// the level whose row count sized the block hash of level L
+__host__ __device__ constexpr int btab_sized_for(int L) { return blocks_are_voxels(L) ? L + 1 : L; }
 struct LevelTabs {
   const unsigned long long* keys[SPS_NUM_LEVELS];
   const int32_t* counts;                 // [SPS_NUM_LEVELS] device voxel counts
-  Slot* btab[SPS_NUM_LEVELS];            // block key -> block id (own hash), or the voxel hash of level L + 2 (from_level)
-  int from_level[SPS_NUM_LEVELS];        // 1: btab[L] is the voxel hash of level L + 2 (its voxels are this level's blocks)
-  int capn[SPS_NUM_LEVELS];              // the table was sized for counts[capn[L]] keys
+  Slot* btab[SPS_NUM_LEVELS];            // block key -> block id (own hash), or the voxel hash of level L + 2 (blocks_are_voxels)
   const int32_t* parent[SPS_NUM_LEVELS]; // fine row -> parent * 8 + k (levels 0..3)
   int32_t* cells[SPS_NUM_LEVELS];        // [blocks][64] voxel rows
   unsigned long long* occ[SPS_NUM_LEVELS];   // [blocks] 64-bit occupancy words
@@ -272,23 +274,24 @@ struct ScratchZero {
   uint32_t* tmask3[SPS_NUM_LEVELS];   // nullptr: level keeps no physical-order tile masks
   uint32_t* sort_hist;                // [4][256] + 4 tile tickets (1028 words), or nullptr: no shape sort this forward
   uint32_t* sort_status;              // [tiles][4][256]
-  int sort_first, sort_levels;
 };
-__device__ __forceinline__ int sort_total(const int32_t* counts, int first, int nlv) {
+// keys of the shape sort: the voxels of all levels (a rolled loop: unrolled, it costs the sort passes 12 registers)
+__device__ __forceinline__ int sort_total(const int32_t* counts) {
   int t = 0;
-  for (int j = 0; j < nlv; ++j) t += counts[first + j];
+#pragma unroll 1
+  for (int j = 0; j < SPS_NUM_LEVELS; ++j) t += counts[j];
   return t;
 }
 __global__ void k_blocks_begin(const LevelTabs T, const ScratchZero z) {
   const int L = blockIdx.y;
   const int n = T.counts[L];
   const uint32_t stride = gridDim.x * blockDim.x, t0 = blockIdx.x * blockDim.x + threadIdx.x;
-  if (T.from_level[L]) {
+  if (blocks_are_voxels(L)) {
     // the blocks are the voxels of level L + 2 and their hash was built by the stride chain: its slots still hold the
     // scan's block-local ranks, so every voxel writes its ROW into its slot (one probe each) -- from here on the table maps
     // a block key to the block id.  Only the occupancy words start from zero: every reader of the cells goes through them.
     const int nb = T.counts[L + 2];
-    const uint32_t mask = table_capacity(T.counts[T.capn[L]]) - 1;
+    const uint32_t mask = table_capacity(T.counts[btab_sized_for(L)]) - 1;
     const unsigned long long* __restrict__ bkeys = T.keys[L + 2];
     Slot* tab = T.btab[L];
     for (uint32_t i = t0; i < (uint32_t)nb; i += stride) {
@@ -311,7 +314,7 @@ __global__ void k_blocks_begin(const LevelTabs T, const ScratchZero z) {
   }
   if (L == 0 && z.sort_hist) {
     for (uint32_t i = t0; i < 1028u; i += stride) z.sort_hist[i] = 0u;
-    const int64_t w = (int64_t)((sort_total(T.counts, z.sort_first, z.sort_levels) + 1023) / 1024) * 1024;
+    const int64_t w = (int64_t)((sort_total(T.counts) + 1023) / 1024) * 1024;
     for (int64_t i = t0; i < w; i += stride) z.sort_status[i] = 0u;
   }
 }
@@ -328,7 +331,7 @@ k_block_insert(const LevelTabs T) {
   // global atomic.  The winner of a block also presets the block's 64 cells and its occupancy word.
   __shared__ int s_cnt, s_base;
   const int L = blockIdx.y;
-  if (T.from_level[L]) return;           // blocks = voxels of level L + 2: nothing to insert
+  if (blocks_are_voxels(L)) return;      // blocks = voxels of level L + 2: nothing to insert
   const int n = T.counts[L];
   const uint32_t mask = table_capacity(n) - 1;
   Slot* tab = T.btab[L];
@@ -369,7 +372,7 @@ __global__ void k_cells_fill(const LevelTabs T) {
   const int n = T.counts[L];
   const uint32_t mask = table_capacity(n) - 1;
   const unsigned long long* keys = T.keys[L];
-  const bool by_parent = T.from_level[L] != 0;
+  const bool by_parent = blocks_are_voxels(L);
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const unsigned long long key = keys[i];
     // block id = the voxel's grandparent row (two reads of the parent arrays), or a lookup in the level's block hash
@@ -381,55 +384,46 @@ __global__ void k_cells_fill(const LevelTabs T) {
   }
 }
 
-// Kernel map of an odd hyper-cube kernel (K0,K0,K0,KT) on tensor stride [2^L]*3+[1] through the
-// block table: thread (o, it) resolves the K0^3 spatial neighbours of voxel o in time plane
-// t + (it - KT/2); k = i0 + K0*(i1 + K0*(i2 + K0*i3)) (ME order), nbr[k][o] coalesced over o.
-template <int K0, int KT>
+// Kernel map of the 5x5x5x1 kernel on level 0 through the block table: thread o resolves the 125 spatial neighbours of
+// voxel o in its own time plane; k = (dx+2) + 5 ((dy+2) + 5 (dz+2)) (ME order), nbr[k][o] coalesced over o.
 __global__ void __launch_bounds__(256)
-k_kernel_map_blk(const unsigned long long* __restrict__ keys, const int32_t* __restrict__ n_ptr,
-                 const Slot* __restrict__ tab, const int32_t* __restrict__ cap_n, const int32_t* __restrict__ cells,
-                 const unsigned long long* __restrict__ occ, int L, int32_t* __restrict__ nbr, int64_t ld,
-                 uint32_t* __restrict__ tile_masks, uint32_t* __restrict__ vmask) {
+k_kernel_map_blk5(const unsigned long long* __restrict__ keys, const int32_t* __restrict__ n_ptr,
+                  const Slot* __restrict__ tab, const int32_t* __restrict__ cap_n, const int32_t* __restrict__ cells,
+                  const unsigned long long* __restrict__ occ, int32_t* __restrict__ nbr, int64_t ld) {
   const int n = *n_ptr;
   if (n == 0) return;
-  constexpr int R = K0 / 2, K3 = K0 * K0 * K0;
   const uint32_t mask = table_capacity(*cap_n) - 1;
-  const int xlim = 1 << (kXBits - L), zlim = 1 << (kZBits - L);
-  const int it = blockIdx.y;   // time plane of the kernel: t + (it - KT/2)
+  const int xlim = 1 << kXBits, zlim = 1 << kZBits;
   const int lane = threadIdx.x & 31;
-  // warps stay converged (o is warp-aligned): the per-tile "offset present" bits come from a ballot
+  // warp-aligned rows (dead lanes past n ride along): ptxas spills 16 bytes for a plain grid-stride loop over o
   for (int o0 = (blockIdx.x * blockDim.x + threadIdx.x) & ~31; o0 < n; o0 += gridDim.x * blockDim.x) {
     const int o = o0 + lane;
     const bool live = o < n;
     const unsigned long long key = live ? keys[o] : 0ull;
-    const int t2 = (int)(key & ((1u << kTBits) - 1)) + it - KT / 2;
-    const bool pok = live && (unsigned)t2 < (1u << kTBits);
-    int32_t* out = nbr + (int64_t)it * K3 * ld + o;
-    const int cx = (int)((key >> kXShift) & ((1u << kXBits) - 1)) >> L;
-    const int cy = (int)((key >> kYShift) & ((1u << kYBits) - 1)) >> L;
-    const int cz = (int)((key >> kZShift) & ((1u << kZBits) - 1)) >> L;
-    const unsigned long long bt = (key & (0xFFull << kBShift)) | (unsigned long long)(unsigned)(pok ? t2 : 0);
+    int32_t* out = nbr + o;
+    const int cx = (int)((key >> kXShift) & ((1u << kXBits) - 1));
+    const int cy = (int)((key >> kYShift) & ((1u << kYBits) - 1));
+    const int cz = (int)((key >> kZShift) & ((1u << kZBits) - 1));
+    const unsigned long long bt = key & ((0xFFull << kBShift) | ((1ull << kTBits) - 1));
     unsigned long long cached_key = kEmptyKey, cached_occ = 0ull;
     const int32_t* cached = nullptr;
-    uint32_t* tm = tile_masks ? tile_masks + 4 * (o0 >> 7) : nullptr;
-    uint32_t present = 0;   // bit k3: neighbour k3 of this time plane exists (K0 = 3: 27 bits)
 #pragma unroll 1
-    for (int dz = -R; dz <= R; ++dz) {
+    for (int dz = -2; dz <= 2; ++dz) {
       const int nz = cz + dz;
-      const bool zok = pok && (unsigned)nz < (unsigned)zlim;
+      const bool zok = (unsigned)nz < (unsigned)zlim;
 #pragma unroll
-      for (int dy = -R; dy <= R; ++dy) {   // (dy, dx) unrolled: up to K0*K0 independent probes in flight per thread
+      for (int dy = -2; dy <= 2; ++dy) {   // (dy, dx) unrolled: up to 25 independent probes in flight per thread
         const int ny = cy + dy;
         const bool yok = zok && (unsigned)ny < (unsigned)xlim;
-        const unsigned long long byz = bt | ((unsigned long long)(unsigned)((ny >> 2) << (L + 2)) << kYShift) |
-                                       ((unsigned long long)(unsigned)((nz >> 2) << (L + 2)) << kZShift);
+        const unsigned long long byz = bt | ((unsigned long long)(unsigned)((ny >> 2) << 2) << kYShift) |
+                                       ((unsigned long long)(unsigned)((nz >> 2) << 2) << kZShift);
         const int lyz = 4 * (ny & 3) + 16 * (nz & 3);
 #pragma unroll
-        for (int dx = -R; dx <= R; ++dx) {
+        for (int dx = -2; dx <= 2; ++dx) {
           const int nx = cx + dx;
           int res = -1;
           if (yok && (unsigned)nx < (unsigned)xlim) {
-            const unsigned long long bkey = byz | ((unsigned long long)(unsigned)((nx >> 2) << (L + 2)) << kXShift);
+            const unsigned long long bkey = byz | ((unsigned long long)(unsigned)((nx >> 2) << 2) << kXShift);
             if (bkey != cached_key) {
               cached_key = bkey;
               const int id = table_find(tab, mask, bkey);
@@ -439,17 +433,10 @@ k_kernel_map_blk(const unsigned long long* __restrict__ keys, const int32_t* __r
             const int l = lyz + (nx & 3);
             if ((cached_occ >> l) & 1ull) res = __ldg(cached + l);
           }
-          const int k3 = (dx + R) + K0 * ((dy + R) + K0 * (dz + R));
-          if (live) out[(int64_t)k3 * ld] = res;
-          if (K3 <= 32 && res >= 0) present |= 1u << (k3 & 31);
-          if (tm) {
-            const int k = it * K3 + k3;
-            if (__any_sync(0xffffffffu, res >= 0) && lane == 0) atomicOr(tm + (k >> 5), 1u << (k & 31));
-          }
+          if (live) out[(int64_t)((dx + 2) + 5 * ((dy + 2) + 5 * (dz + 2))) * ld] = res;
         }
       }
     }
-    if (vmask && live) vmask[(int64_t)o * 4 + it] = present;
   }
 }
 
@@ -457,26 +444,25 @@ k_kernel_map_blk(const unsigned long long* __restrict__ keys, const int32_t* __r
 // and, per axis, in at most ONE adjacent block (when the voxel sits on that face), i.e. in 1, 2, 4 or 8 blocks
 // (3.4 on average).  Each thread first resolves those blocks (independent hash probes, all in flight), parks
 // block id + occupancy word in shared memory, then answers the 27 lookups with a bit test and, for present
-// neighbours only, one 4-byte read.  (The generic kernel above re-probes whenever the block changes along
-// x: ~13 probes per thread; this was the dominant kernel after the convolutions were sped up.)
+// neighbours only, one 4-byte read.  (Probing like the 5x5x5 kernel above, again whenever the block changes along x, took
+// ~13 probes per thread; this was the dominant kernel after the convolutions were sped up.)
 struct KmapOut {
   int32_t* nbr[SPS_NUM_LEVELS];           // [81][ld] per level
   uint32_t* tile_masks[SPS_NUM_LEVELS];   // physical-order tile masks, or nullptr (shape-sorted level of the fused forward)
   uint32_t* vmask[SPS_NUM_LEVELS];        // [ld][4] per-voxel 27-bit presence words of the three time planes (+ pad): one 16-byte line
   int64_t ld;
-  int dense_mask;                         // bit L: level L stores absent entries (-1) too
+  int dense;                              // absent entries (-1) are stored too
   // shape sort fused in (nullptr: no sort this forward): the voxel's sort key, its row number and the digit histograms of
   // the four radix passes leave this kernel, so the presence words are not read back by a separate key pass
   uint32_t* sort_keys; int32_t* sort_vals; uint32_t* sort_hist;
-  int sort_first, sort_last;
 };
-// All levels in one launch: blockIdx.z = level, blockIdx.y = time plane of the kernel.
+// All levels in one launch: blockIdx.z = level; a thread walks the three time planes of the kernel.
 // (capping this kernel at 32 registers to fit more blocks beside another lane's convolution CTA made it 1.5x slower
 // and the step 18 % slower: profiles/r2_experiments.md)
 __device__ __forceinline__ uint32_t shape_bits(uint32_t pat);
-template <int KT>
 __global__ void __launch_bounds__(256, 6)
 k_kernel_map_blk3(const LevelTabs T, const KmapOut O) {
+  constexpr int KT = 3;   // time planes of the kernel
   __shared__ int sId[8][256];
   __shared__ unsigned long long sOcc[8][256];
   const int L = blockIdx.z;
@@ -490,17 +476,17 @@ k_kernel_map_blk3(const LevelTabs T, const KmapOut O) {
   uint32_t* __restrict__ tile_masks = O.tile_masks[L];
   uint32_t* __restrict__ vmask = O.vmask[L];
   const int64_t ld = O.ld;
-  const int dense = (O.dense_mask >> L) & 1;
-  const uint32_t mask = table_capacity(T.counts[T.capn[L]]) - 1;
+  const int dense = O.dense;
+  const uint32_t mask = table_capacity(T.counts[btab_sized_for(L)]) - 1;
   const int xlim = 1 << (kXBits - L), zlim = 1 << (kZBits - L);
   const int tid = threadIdx.x, lane = tid & 31;
   const uint32_t planes = (uint32_t)*T.tplanes;
-  const bool sorting = O.sort_keys != nullptr && L >= O.sort_first && L <= O.sort_last;
+  const bool sorting = O.sort_keys != nullptr;
   __shared__ uint32_t s_hist[4][256];
   int sort_off = 0;
   if (sorting) {
     for (int i = tid; i < 1024; i += blockDim.x) (&s_hist[0][0])[i] = 0u;
-    for (int q = O.sort_first; q < L; ++q) sort_off += T.counts[q];
+    for (int q = 0; q < L; ++q) sort_off += T.counts[q];
     __syncthreads();
   }
   for (int o0 = (blockIdx.x * blockDim.x + tid) & ~31; o0 < n; o0 += gridDim.x * blockDim.x) {
@@ -605,7 +591,7 @@ k_kernel_map_blk3(const LevelTabs T, const KmapOut O) {
       // one offset more, not their whole difference (offsets walked per tile -3..4 %, tools/tile_stats.py)
       uint32_t g = shape_bits(por) | (has_lo << 27) | (has_hi << 28);
       g ^= g >> 1; g ^= g >> 2; g ^= g >> 4; g ^= g >> 8; g ^= g >> 16;
-      const uint32_t skey = g | ((uint32_t)(L - O.sort_first) << 29);
+      const uint32_t skey = g | ((uint32_t)L << 29);
       O.sort_keys[sort_off + o] = skey;
       O.sort_vals[sort_off + o] = o;
 #pragma unroll
@@ -635,12 +621,9 @@ k_kernel_map_blk3(const LevelTabs T, const KmapOut O) {
 // keys are produced, and a tile learns the number of equal digits in the tiles before it by decoupled look-back over
 // per-tile status words (aggregate / inclusive-prefix flags in the top two bits).  Round 1 ran 13 launches per level.
 struct SortArgs {
-  const uint32_t* vmask[SPS_NUM_LEVELS];
   int32_t* perm[SPS_NUM_LEVELS];
   const int32_t* counts;
   int32_t* status;      // sticky status word of the context (a look-back that never completes is reported, not waited for)
-  int64_t ld;
-  int first, nlv;
 };
 constexpr int kSortThreads = 256, kSortItems = 8, kSortTile = kSortThreads * kSortItems;
 constexpr uint32_t kOsAggregate = 1u << 30, kOsPrefix = 2u << 30, kOsValue = (1u << 30) - 1u;
@@ -678,7 +661,7 @@ k_onesweep_pass(const SortArgs A, const uint32_t* __restrict__ keys, const int32
   __shared__ int s_base[256];                   // global position of this tile's first element per digit
   __shared__ int s_scan[kWarps];
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
-  const int n = sort_total(A.counts, A.first, A.nlv);
+  const int n = sort_total(A.counts);
   const int ntiles = (n + kSortTile - 1) / kSortTile;
   // the grid is sized by the host bound (rows x levels): the surplus blocks leave before touching anything, the first
   // ntiles blocks take one ticket each
@@ -760,9 +743,10 @@ k_onesweep_pass(const SortArgs A, const uint32_t* __restrict__ keys, const int32
     const int pos = s_base[digit] + wcount[r * kWarps + w][digit] + rank[r];
     if (LAST) {
       const int j = (int)(key[r] >> 29);
-      int off = 0;
-      for (int q = 0; q < j; ++q) off += A.counts[A.first + q];
-      A.perm[A.first + j][pos - off] = val[r];
+      int off = 0;   // (a predicated sum: with a loop to j the kernel takes 64 registers instead of 48)
+#pragma unroll
+      for (int q = 0; q < SPS_NUM_LEVELS - 1; ++q) if (q < j) off += A.counts[q];
+      A.perm[j][pos - off] = val[r];
     } else {
       keys_out[pos] = key[r];
       vals_out[pos] = val[r];
@@ -770,10 +754,9 @@ k_onesweep_pass(const SortArgs A, const uint32_t* __restrict__ keys, const int32
   }
 }
 
-// present-offset masks of the 128-row tiles taken in `perm` order, and (slices != nullptr) the tiles' slices of
-// the kernel map gathered once for all the convolutions of the level: slices[tile][e][r] = input row
-// of sorted row r under the tile's e-th present offset, entry e = #present = the tile's own rows.
-// All sorted levels in one launch (blockIdx.y).
+// present-offset masks of the 128-row tiles taken in `perm` order, and the tiles' slices of the kernel map gathered once
+// for all the convolutions of the level: slices[tile][e][r] = input row of sorted row r under the tile's e-th present
+// offset, entry e = #present = the tile's own rows.  All levels in one launch (blockIdx.y).
 struct SliceArgs {
   const uint32_t* vmask[SPS_NUM_LEVELS];
   const int32_t* perm[SPS_NUM_LEVELS];
@@ -782,11 +765,10 @@ struct SliceArgs {
   int32_t* slices[SPS_NUM_LEVELS];
   const int32_t* counts;
   int64_t ld;
-  int first;
 };
 __global__ void __launch_bounds__(128)
 k_tile_masks_perm(const SliceArgs A) {
-  const int L = A.first + blockIdx.y;
+  const int L = blockIdx.y;
   const int n = A.counts[L];
   const int ntiles = (n + 127) / 128;
   const uint32_t* __restrict__ vmask = A.vmask[L];
@@ -818,36 +800,33 @@ k_tile_masks_perm(const SliceArgs A) {
                             m[0][2] | m[1][2] | m[2][2] | m[3][2]};
     if (threadIdx.x < 3) masks[4 * tile + threadIdx.x] = tm[threadIdx.x];
     if (threadIdx.x == 3) masks[4 * tile + 3] = 0;
-    if (slices) {
-      const int nact = __popc(tm[0]) + __popc(tm[1]) + __popc(tm[2]);
-      if (threadIdx.x < 96) {
-        const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-        if ((tm[w] >> l) & 1u) {
-          const int before = (w > 0 ? __popc(tm[0]) : 0) + (w > 1 ? __popc(tm[1]) : 0) + __popc(tm[w] & ((1u << l) - 1u));
-          klist[before] = (uint8_t)threadIdx.x;
-        }
+    const int nact = __popc(tm[0]) + __popc(tm[1]) + __popc(tm[2]);
+    if (threadIdx.x < 96) {
+      const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+      if ((tm[w] >> l) & 1u) {
+        const int before = (w > 0 ? __popc(tm[0]) : 0) + (w > 1 ? __popc(tm[1]) : 0) + __popc(tm[w] & ((1u << l) - 1u));
+        klist[before] = (uint8_t)threadIdx.x;
       }
-      __syncthreads();
-      int32_t* dst = slices + (int64_t)tile * (SPS_TILE_SLICE_ENTRIES * 128) + threadIdx.x;
-      const uint32_t mine[3] = {w0, w1, w2};
-      // SPS_SLICE_BATCH (16) entries at a time: the loads of a batch are issued before the first store (the pass waits on these random
-      // 4-byte reads; unroll depth = reads in flight per thread)
-      static_assert(SPS_SLICE_BATCH >= 1, "");
-      for (int e0 = 0; e0 < nact; e0 += SPS_SLICE_BATCH) {
-        int val[SPS_SLICE_BATCH];
-#pragma unroll
-        for (int u = 0; u < SPS_SLICE_BATCH; ++u) {
-          const int e = e0 + u;
-          const int k = e < nact ? klist[e] : 0;
-          val[u] = -1;
-          if (e < nact && ((mine[k >> 5] >> (k & 31)) & 1u)) val[u] = __ldg(nbr + (int64_t)k * ld + v);
-        }
-#pragma unroll
-        for (int u = 0; u < SPS_SLICE_BATCH; ++u)
-          if (e0 + u < nact) dst[(e0 + u) * 128] = val[u];
-      }
-      dst[nact * 128] = v;
     }
+    __syncthreads();
+    int32_t* dst = slices + (int64_t)tile * (SPS_TILE_SLICE_ENTRIES * 128) + threadIdx.x;
+    const uint32_t mine[3] = {w0, w1, w2};
+    // kSliceBatch entries at a time: the loads of a batch are issued before the first store (the pass waits on these random
+    // 4-byte reads; unroll depth = reads in flight per thread)
+    for (int e0 = 0; e0 < nact; e0 += kSliceBatch) {
+      int val[kSliceBatch];
+#pragma unroll
+      for (int u = 0; u < kSliceBatch; ++u) {
+        const int e = e0 + u;
+        const int k = e < nact ? klist[e] : 0;
+        val[u] = -1;
+        if (e < nact && ((mine[k >> 5] >> (k & 31)) & 1u)) val[u] = __ldg(nbr + (int64_t)k * ld + v);
+      }
+#pragma unroll
+      for (int u = 0; u < kSliceBatch; ++u)
+        if (e0 + u < nact) dst[(e0 + u) * 128] = val[u];
+    }
+    dst[nact * 128] = v;
     __syncthreads();
   }
 }
@@ -1068,23 +1047,6 @@ int build_maps_impl(sps_ctx* ctx, const Conv0Fused* c0, cudaStream_t st);
 // exact-fp32 mode gathers from the dense maps (generic CUDA-core kernels)
 static inline bool needs_dense_maps(const sps_ctx* ctx) { return ctx->backend == SPS_BACKEND_FP32; }
 
-#ifndef SPS_TILE_SLICES
-#define SPS_TILE_SLICES 1
-#endif
-static const int g_tile_slices = SPS_TILE_SLICES;   // gather the kernel map per sorted tile once per level
-#ifndef SPS_BLOCKS_FROM_LEVELS
-#define SPS_BLOCKS_FROM_LEVELS 1
-#endif
-static const int g_blocks_from_levels = SPS_BLOCKS_FROM_LEVELS;   // block tables of levels 0..2 = voxel hashes of levels 2..4
-#ifndef SPS_FIRST_SORTED_LEVEL
-#define SPS_FIRST_SORTED_LEVEL 0
-#endif
-constexpr int kFirstSortedLevel = SPS_FIRST_SORTED_LEVEL;
-#ifndef SPS_LAST_SORTED_LEVEL
-#define SPS_LAST_SORTED_LEVEL 4     // all levels ride in the one concatenated sort (level 4 adds 2 % to its keys)
-#endif
-constexpr int kLastSortedLevel = SPS_LAST_SORTED_LEVEL;
-constexpr int kSortedLevels = kLastSortedLevel - kFirstSortedLevel + 1;
 constexpr int64_t kMinRowsForSort = 400000;   // small inputs (single scans) are launch-bound: the sort does not pay
 
 static inline bool sort_active(const sps_ctx* ctx) {
@@ -1092,16 +1054,16 @@ static inline bool sort_active(const sps_ctx* ctx) {
 }
 
 // perm[L] = voxel rows of level L sorted by neighbourhood-shape key, ptmask[L] = tile masks in that order, tslice[L] = the
-// kernel map gathered per sorted tile -- for all sorted levels at once: 1 + 4 + 1 launches.
+// kernel map gathered per sorted tile -- for all levels at once (level 4 adds 2 % to the keys): 4 + 1 launches.
 static int pattern_order(sps_ctx* ctx, cudaStream_t st) {
   if (!sort_active(ctx)) return SPS_OK;
   const int64_t n = ctx->n > 0 ? ctx->n : 1;
   SortArgs A;
-  for (int L = 0; L < SPS_NUM_LEVELS; ++L) { A.vmask[L] = ctx->vmask[L]; A.perm[L] = ctx->perm[L]; }
-  A.counts = ctx->counts; A.status = ctx->status; A.ld = ctx->ld; A.first = kFirstSortedLevel; A.nlv = kSortedLevels;
+  for (int L = 0; L < SPS_NUM_LEVELS; ++L) A.perm[L] = ctx->perm[L];
+  A.counts = ctx->counts; A.status = ctx->status;
   uint32_t* hist = ctx->sort_hist;
   // (keys, row numbers and digit histograms were left behind by the 3x3x3x3 kernel-map pass)
-  const int tiles_max = cdiv(n * kSortedLevels, kSortTile);
+  const int tiles_max = cdiv(n * SPS_NUM_LEVELS, kSortTile);
   for (int pass = 0; pass < 4; ++pass) {
     const uint32_t* ki = ctx->sort_keys[pass & 1];
     const int32_t* vi = ctx->sort_vals[pass & 1];
@@ -1118,10 +1080,10 @@ static int pattern_order(sps_ctx* ctx, cudaStream_t st) {
   SliceArgs S;
   for (int L = 0; L < SPS_NUM_LEVELS; ++L) {
     S.vmask[L] = ctx->vmask[L]; S.perm[L] = ctx->perm[L]; S.masks[L] = ctx->ptmask[L]; S.nbr[L] = ctx->nbr3[L];
-    S.slices[L] = g_tile_slices ? ctx->tslice[L] : nullptr;
+    S.slices[L] = ctx->tslice[L];
   }
-  S.counts = ctx->counts; S.ld = ctx->ld; S.first = kFirstSortedLevel;
-  k_tile_masks_perm<<<dim3(grid_for(n / 128 + 1, 1, 148 * 8), kSortedLevels), 128, 0, st>>>(S);
+  S.counts = ctx->counts; S.ld = ctx->ld;
+  k_tile_masks_perm<<<dim3(grid_for(n / 128 + 1, 1, 148 * 8), SPS_NUM_LEVELS), 128, 0, st>>>(S);
   prof_mark(ctx, "slices", st);
   SPS_CUDA_CHECK(cudaGetLastError());
   ctx->forward_launches += 5;
@@ -1145,7 +1107,7 @@ int sps::build_maps_impl(sps_ctx* ctx, const Conv0Fused* c0, cudaStream_t st) {
     // The voxels of level L are the 4x4x4-cell blocks of level L - 2: levels 2..4 build their hash where the block table
     // of that level lives, so that it answers "block key -> block row" later without a second hash build
     // (k_block_insert was 100 us per forward); k_blocks_begin writes the rows into the slots.
-    Slot* tab = (g_blocks_from_levels && L >= 2) ? ctx->btab[L - 2] : ctx->table;
+    Slot* tab = L >= 2 ? ctx->btab[L - 2] : ctx->table;
     int32_t* sums = ctx->block_sums;
     k_level_begin<<<grid_for(table_capacity(n), 256), 256, 0, st>>>(tab, n_fine, -1, nullptr, ctx->child[L], ctx->ld, nullptr,
                                                                     ctx->up_cls + 16 * (L - 1));
@@ -1166,33 +1128,24 @@ int sps::build_maps_impl(sps_ctx* ctx, const Conv0Fused* c0, cudaStream_t st) {
     prof_mark(ctx, "up_order", st);
   }
   // ---- 2. block tables of all five levels (three launches) ----
-  // fused forward on a shape-sorted level: the convolutions read the tile slices and the sorted tile masks, the slices
-  // read only present entries -> neither the -1 entries nor the physical-order tile masks are produced
+  // fused forward with the shape sort: the convolutions read the tile slices and the sorted tile masks, the slices read
+  // only present entries -> neither the -1 entries nor the physical-order tile masks are produced
   const bool sorting = sort_active(ctx);
-  auto sparse_ok = [&](int L) {
-    return c0 != nullptr && !needs_dense_maps(ctx) && g_tile_slices && ctx->tslice[L] != nullptr && sorting && L >= kFirstSortedLevel &&
-           L <= kLastSortedLevel;
-  };
+  const bool sparse = c0 != nullptr && !needs_dense_maps(ctx) && sorting;
   LevelTabs T;
   ScratchZero Z;
   KmapOut O;
-  O.dense_mask = 0;
   for (int L = 0; L < SPS_NUM_LEVELS; ++L) {
     T.keys[L] = ctx->keys[L]; T.btab[L] = ctx->btab[L]; T.cells[L] = ctx->bcells[L]; T.occ[L] = ctx->bocc[L];
-    const bool from_level = g_blocks_from_levels && L + 2 < SPS_NUM_LEVELS;
-    T.from_level[L] = from_level ? 1 : 0;
-    T.capn[L] = from_level ? L + 1 : L;      // level L + 2's hash was sized for the rows of level L + 1
     T.parent[L] = ctx->parent[L];
-    Z.tmask3[L] = sparse_ok(L) ? nullptr : ctx->tmask3[L];
+    Z.tmask3[L] = sparse ? nullptr : ctx->tmask3[L];
     O.nbr[L] = ctx->nbr3[L]; O.tile_masks[L] = Z.tmask3[L]; O.vmask[L] = ctx->vmask[L];
-    if (!sparse_ok(L)) O.dense_mask |= 1 << L;
   }
   T.counts = ctx->counts; T.nblocks = ctx->nblocks; T.tplanes = ctx->tplanes;
   Z.sort_hist = sorting ? ctx->sort_hist : nullptr; Z.sort_status = ctx->sort_status;
-  Z.sort_first = kFirstSortedLevel; Z.sort_levels = kSortedLevels;
   O.ld = ctx->ld;
+  O.dense = sparse ? 0 : 1;
   O.sort_keys = sorting ? ctx->sort_keys[0] : nullptr; O.sort_vals = ctx->sort_vals[0]; O.sort_hist = ctx->sort_hist;
-  O.sort_first = kFirstSortedLevel; O.sort_last = kLastSortedLevel;
   const int gx = grid_for(n, 256, 148 * 6);   // one wave of the kernel-map pass (6 blocks of 256 threads per SM at 40 registers)
   k_blocks_begin<<<dim3(grid_for(table_capacity(n), 256, 148 * 8), SPS_NUM_LEVELS), 256, 0, st>>>(T, Z);
   k_block_insert<<<dim3(gx, SPS_NUM_LEVELS), 256, 0, st>>>(T);
@@ -1201,31 +1154,28 @@ int sps::build_maps_impl(sps_ctx* ctx, const Conv0Fused* c0, cudaStream_t st) {
   // ---- 3. conv0 off the level-0 block table (fused forward), or the 5x5x5x1 table (layer-level API) ----
   if (c0) {
     if (c0->feat)   // per-voxel features: gather them through the block table
-      k_conv0_blk<<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + T.capn[0], ctx->bcells[0], ctx->bocc[0], c0->feat,
+      k_conv0_blk<<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + btab_sized_for(0), ctx->bcells[0], ctx->bocc[0], c0->feat,
                                                      c0->w, c0->shift, c0->round_out, c0->out, c0->out_ld);
     else            // one constant feature (SPSModel.forward): presence bits only
-      k_conv0_const<<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + T.capn[0], ctx->bocc[0], c0->cfeat,
+      k_conv0_const<<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + btab_sized_for(0), ctx->bocc[0], c0->cfeat,
                                                        c0->w, c0->shift, c0->round_out, c0->out, c0->out_ld);
     prof_mark(ctx, "conv0+kmap5", st);
   } else {
-    k_kernel_map_blk<5, 1><<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + T.capn[0], ctx->bcells[0], ctx->bocc[0], 0,
-                                                              ctx->nbr5, ctx->ld, nullptr, nullptr);
+    k_kernel_map_blk5<<<grid_for(n, 256), 256, 0, st>>>(ctx->keys[0], ctx->counts + 0, ctx->btab[0], ctx->counts + btab_sized_for(0), ctx->bcells[0],
+                                                         ctx->bocc[0], ctx->nbr5, ctx->ld);
     prof_mark(ctx, "kmap5.L0", st);
   }
   ctx->have_nbr5 = c0 == nullptr;
   // ---- 4. 3x3x3x3 kernel maps of all five levels (one launch: level x time plane) ----
-  k_kernel_map_blk3<3><<<dim3(gx, 1, SPS_NUM_LEVELS), 256, 0, st>>>(T, O);
+  k_kernel_map_blk3<<<dim3(gx, 1, SPS_NUM_LEVELS), 256, 0, st>>>(T, O);
   prof_mark(ctx, "kmap3", st);
   SPS_CUDA_CHECK(cudaGetLastError());
   ctx->forward_launches += 16 + 1 + 3 + 1 + 1;
-  // ---- 5. shape sort + per-tile slices of the sorted levels ----
+  // ---- 5. shape sort + per-tile slices ----
   { const int rc = pattern_order(ctx, st); if (rc != SPS_OK) return rc; }
   ctx->have_maps = true;
-  ctx->dense_maps = O.dense_mask == (1 << SPS_NUM_LEVELS) - 1;
+  ctx->dense_maps = !sparse;
   ctx->have_perm = sorting;
-  ctx->have_slices = ctx->have_perm && g_tile_slices && ctx->tslice[kLastSortedLevel] != nullptr;
-  ctx->first_sorted = kFirstSortedLevel;
-  ctx->last_sorted = kLastSortedLevel;
   return SPS_OK;
 }
 

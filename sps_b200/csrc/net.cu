@@ -177,7 +177,7 @@ extern "C" int sps_net_finalize(sps_net* net, void* d_weights, size_t bytes, voi
     // channels: two K segments (1.5 stages per offset instead of 2; measured 135 -> 121 us).  The 32 + 16 and 16 + 8
     // buffers of block6 / block7 stay one padded segment: splitting them fetches every row twice and the gather is bound
     // by rows, not bytes (block7.conv1 119 -> 132 us with the split).
-    const int seg = (!tail && cin > cout && cout == 64 && !getenv("SPS_NO_CIN_SPLIT")) ? cout : 0;
+    const int seg = (!tail && cin > cout && cout == 64) ? cout : 0;
     if (!add_conv(net->blk1[b], name + ".0.conv1.kernel", name + ".0.norm1", 81, cin, cout, tail, false, seg)) return false;
     std::vector<float> w; std::vector<double> sh;
     if (!fold_conv(net, name + ".0.conv2.kernel", name + ".0.norm2", 81, cout, cout, w, sh)) return false;
@@ -322,12 +322,11 @@ static int run_conv(sps_ctx* c, const ConvIo& io, const char* name, const ConvW&
   return rc;
 }
 
-// processing order of the 3x3x3x3 convs at level L: rows in neighbourhood-shape order where the level was sorted,
+// processing order of the 3x3x3x3 convs at level L: rows in neighbourhood-shape order when the maps were sorted,
 // otherwise physical order; both kinds of tile masks exist.
 static ConvIo io3(const sps_ctx* c, int L) {
-  const bool pm = c->have_perm && L >= c->first_sorted && L <= c->last_sorted;
-  return ConvIo{pm ? c->ptmask[L] : c->tmask3[L], pm ? c->perm[L] : nullptr, pm && c->have_slices ? c->tslice[L] : nullptr,
-                SPS_CONV_NBR, c->nbr3[L]};
+  const bool pm = c->have_perm;
+  return ConvIo{pm ? c->ptmask[L] : c->tmask3[L], pm ? c->perm[L] : nullptr, pm ? c->tslice[L] : nullptr, SPS_CONV_NBR, c->nbr3[L]};
 }
 
 int unet_forward(sps_ctx* c, const sps_net* net, const float* feat0, float* logits, cudaStream_t st,

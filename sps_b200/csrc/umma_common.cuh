@@ -28,15 +28,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
       "}\n" ::"r"(bar), "r"(parity)
       : "memory");
 }
-#ifdef SPS_CP_CG
-#define SPS_CP_ASYNC16 "cp.async.cg.shared.global [%0], [%1], 16, %2;"
-#else
-#define SPS_CP_ASYNC16 "cp.async.ca.shared.global [%0], [%1], 16, %2;"
-#endif
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32_t src_bytes) {
-  asm volatile(SPS_CP_ASYNC16 ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
@@ -93,11 +84,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float* v) {
                : "r"(taddr));
 #pragma unroll
   for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-__device__ __forceinline__ float round_tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return __uint_as_float(r);
 }
 
 // groups (of 4 channels) reserved per kernel offset in the K-major weight matrix / the stage plan

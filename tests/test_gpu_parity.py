@@ -288,6 +288,37 @@ def test_generic_unet_entry_matches_fused_forward(engine_mod, state_dict):
     assert np.abs(got - ref).max() < 5e-5
 
 
+def test_level_views_after_sorted_and_unsorted_passes(engine_mod, state_dict):
+    """What sps_ctx_level hands out at every level: the dense 3x3x3x3 table after an unsorted forward, only the
+    shape-sorted processing order (perm, tile masks, tile slices) after a sorted fused forward on the default backend,
+    the table again after sps_build_maps, and both after a sorted forward on the exact fp32 backend."""
+    rows = make_case("tiny", seed=3)
+    pts = dev(rows[:, :5])
+    net = engine_mod.Net(state_dict)
+    eng = engine_mod.Engine(len(pts))
+
+    def views():
+        eng.status()
+        return [eng.level(L) for L in range(5)]
+
+    eng.set_conv_backend(0)
+    eng.set_pattern_sort(0)
+    eng.forward(net, pts, 0.1)
+    for L, v in enumerate(views()):
+        assert v.nbr3 and not v.perm and not v.tile_mask and not v.tile_slices, L
+    eng.set_pattern_sort(2)
+    eng.forward(net, pts, 0.1)
+    for L, v in enumerate(views()):
+        assert not v.nbr3 and v.perm and v.tile_mask and v.tile_slices, L
+    eng.build_maps()
+    for L, v in enumerate(views()):
+        assert v.nbr3 and v.perm and v.tile_mask and v.tile_slices, L
+    eng.set_conv_backend(1)
+    eng.forward(net, pts, 0.1)
+    for L, v in enumerate(views()):
+        assert v.nbr3 and v.perm and v.tile_mask and v.tile_slices, L
+
+
 @pytest.mark.tensor_path
 def test_scan_streamer_graph_replay_matches_eager_call(engine_mod, state_dict):
     """ScanStreamer: the per-scan loop of sps_node.py:111-120 (prune -> assemble -> forward) captured once as a CUDA graph.

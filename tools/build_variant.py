@@ -1,5 +1,5 @@
-"""Build an experimental variant of libsps_b200.so (extra -D flags) next to the product library:
-    python tools/build_variant.py NAME -DSPS_V6_S16=4 ...   ->  sps_b200/variants/libsps_NAME.so
+"""Build an experimental variant of libsps_b200.so (extra nvcc flags) next to the product library:
+    python tools/build_variant.py NAME -Xptxas -maxrregcount=64 ...   ->  sps_b200/variants/libsps_NAME.so
 Select it at run time with SPS_B200_LIB=sps_b200/variants/libsps_NAME.so (A/B measurements only)."""
 import os, subprocess, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

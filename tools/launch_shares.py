@@ -18,7 +18,7 @@ n = len(seq) // 2                                   # two forwards were captured
 fwd = seq[n:]
 groups = [("`k_conv_umma6<*>` (all instantiations)", lambda k: k.startswith("k_conv_umma6"),
            [k for k in st if k.startswith(("conv1", "conv2", "conv3", "conv4", "convtr", "block")) and k != "blocks"]),
-          ("`k_kernel_map_blk3<3>`", lambda k: k.startswith("k_kernel_map_blk3"), ["kmap3"]),
+          ("`k_kernel_map_blk3`", lambda k: k.startswith("k_kernel_map_blk3"), ["kmap3"]),
           ("shape sort (4 x `k_onesweep_pass`; the keys come out of the kernel-map pass)", lambda k: k.startswith("k_onesweep"), ["sort"]),
           ("`k_tile_masks_perm`", lambda k: k.startswith("k_tile_masks_perm"), ["slices"]),
           ("`k_conv0_const`", lambda k: k.startswith("k_conv0"), ["conv0+kmap5"]),
