@@ -80,25 +80,37 @@ def merge_rows(x2: torch.Tensor) -> torch.Tensor:
     return (g[:, :, 0] + g[:, :, 1]).reshape(V, C2 // 2)
 
 
+def _addr(x):
+    """Device address of a CUDA tensor, or a raw device pointer (an ``Engine.level`` view field) as it is; None -> NULL."""
+    if x is None or isinstance(x, int):
+        return x
+    return x.data_ptr()
+
+
 def kernel_map_tile_masks(map, map_ld, K, n_out, n_out_max):
-    """Present-offset bitmask per 128-row tile of a dense kernel map (tensor-core path input)."""
+    """Present-offset bitmask per 128-row tile of a dense kernel map (tensor-core path input).  ``map``: a CUDA tensor
+    or a device pointer."""
     lib = _cabi.load()
-    masks = torch.zeros(((n_out_max + 127) // 128 + 1, 4), dtype=torch.int32, device=map.device)
-    check(lib.sps_kernel_map_tile_masks(_ptr(map), int(map_ld), int(K), _ptr(n_out), int(n_out_max), _ptr(masks), _stream()),
-          "sps_kernel_map_tile_masks")
+    masks = torch.zeros(((n_out_max + 127) // 128 + 1, 4), dtype=torch.int32, device=n_out.device)
+    check(lib.sps_kernel_map_tile_masks(C.c_void_p(_addr(map)), int(map_ld), int(K), _ptr(n_out), int(n_out_max), _ptr(masks),
+                                        _stream()), "sps_kernel_map_tile_masks")
     return masks
 
 
 def conv_fwd(inp, weight, n_out, *, map=None, map_ld=0, mode=_cabi.SPS_CONV_NBR, shift=None, in2=None, weight2=None,
              res=None, relu=False, out=None, head_w=None, head_b=0.0, head_out=None, weight_kmajor=None,
-             round_out=False, n_out_max=None, backend=None, tile_mask=None, io_f16=False, flags=0, cin_rows=None, cin2_rows=None, cin_split=0):
+             round_out=False, n_out_max=None, backend=None, tile_mask=None, io_f16=False, flags=0, cin_rows=None, cin2_rows=None, cin_split=0,
+             perm=None, tile_slices=None):
     """out[o] = act(sum_k in[map[k][o]] @ W[k] (+ in2[o] @ W2) + shift (+ res[o])); ``n_out`` is a
     1-element int32 CUDA tensor (device-side count).  ``inp``/``out``/``in2``/``res`` may be
     channel slices (stride(0) is the leading dimension).  ``io_f16``: ``inp``/``in2``/``res``/``out`` are fp16
     rows and ``weight_kmajor`` comes from :func:`pack_kmajor_f16` (SPS_IO_F16, the fused forward's format).
     ``flags``: SPS_CONV_FOLD_LO / SPS_CONV_OUT_SPLIT; ``cin_rows`` / ``cin2_rows``: channel counts the kernel sees when the rows are
     hi|lo pairs (2 x the weight's).  ``backend``: SPS_BACKEND_* of this one call (default AUTO) -- the library has no
-    process-wide switch."""
+    process-wide switch.  ``perm`` / ``tile_mask`` / ``tile_slices``: a processing order of the output rows, the tile
+    masks in that order and, optionally, the kernel map gathered per tile (``map`` may then be None) -- what
+    ``Engine.level`` hands out after a shape-sorted pass.  ``map``, ``tile_mask``, ``perm`` and ``tile_slices`` take CUDA
+    tensors or raw device pointers."""
     lib = _cabi.load()
     K = weight.shape[0] if weight.dim() == 3 else 1
     cin, cout = weight.shape[-2], weight.shape[-1]
@@ -109,7 +121,7 @@ def conv_fwd(inp, weight, n_out, *, map=None, map_ld=0, mode=_cabi.SPS_CONV_NBR,
         out = torch.empty((max(n_out_max, 1), width), dtype=torch.float16 if io_f16 else torch.float32, device=inp.device)
     a = _cabi.ConvArgs()
     a.mode, a.K, a.cin, a.cout = mode, K, cin, cout
-    a.map, a.map_ld = (map.data_ptr() if map is not None else None), int(map_ld)
+    a.map, a.map_ld = _addr(map), int(map_ld)
     a.n_out, a.n_out_max = n_out.data_ptr(), int(n_out_max)
     a.in_, a.in_ld = inp.data_ptr(), inp.stride(0)
     a.weight = weight.data_ptr()
@@ -134,10 +146,9 @@ def conv_fwd(inp, weight, n_out, *, map=None, map_ld=0, mode=_cabi.SPS_CONV_NBR,
         a.cin = int(cin_rows)
     if cin2_rows is not None:
         a.cin2 = int(cin2_rows)
-    if weight_kmajor is not None and map is not None and tile_mask is None and K <= 81:
+    if weight_kmajor is not None and map is not None and tile_mask is None and perm is None and K <= 81:
         tile_mask = kernel_map_tile_masks(map, map_ld, K, n_out, n_out_max)
-    if tile_mask is not None:
-        a.tile_mask = tile_mask.data_ptr()
+    a.tile_mask, a.perm, a.tile_slices = _addr(tile_mask), _addr(perm), _addr(tile_slices)
     with torch.cuda.device(inp.device):
         check(lib.sps_conv_fwd(C.byref(a), _stream()), "sps_conv_fwd")
     return out if out is not None else head_out
