@@ -136,8 +136,9 @@ def spread_state_dict(sd, pts, gain=8.0, voxel=0.1):
 @pytest.mark.tensor_path
 @pytest.mark.parametrize("sensor,seed,submap", [("tiny", 3, "voxel"), ("hdl-32", 2, "voxel"), ("os1-64", 0, "radius")])
 def test_scores_match_oracle(engine_mod, state_dict, sensor, seed, submap):
-    """Default arithmetic (tcgen05 on fp16 rows + exact-fp32 FMA kernels on the 8-channel layers, fp32 level-0 tail)
-    against the fp32 oracle at the north-star bar: 2e-3 on the scores, >= 99.9 % equal labels -- on the contract
+    """Default arithmetic (tcgen05 on fp16 rows for every layer but conv0; the 8-output-channel layers fold the low parts
+    of their weights into spare accumulator columns; the level-0 concat buffer is stored as fp16 hi|lo pairs) against
+    the fp32 oracle at the north-star bar: 2e-3 on the scores, >= 99.9 % equal labels -- on the contract
     network AND on weights whose scores spread over (0,1) and straddle eps (1x tolerance for both)."""
     rows = make_case(sensor, seed=seed, submap=submap, n_map_poses=6)
     pts = rows[:, :5]
