@@ -252,6 +252,35 @@ int sps_infer_scan(sps_ctx* ctx, const sps_net* net, const sps_map* map, const f
                    int64_t n_scan, float voxel_size, float* d_scores, void* d_scratch,
                    size_t scratch_bytes, int32_t* d_counts, void* stream);
 
+/* A batch of deployment scans in one call: util.prune (sps_submap_crop_voxel) + util.infer's assembly per scan,
+ * collated.  d_scans fp32 [n_total, ld >= 3] = x, y, z (further columns are ignored) of `batch` scans already in the
+ * map frame, concatenated; h_offsets (HOST) int64 [batch + 1]: scan b = rows h_offsets[b] .. h_offsets[b+1], with
+ * h_offsets[0] == 0, non-decreasing, n_total = h_offsets[batch] <= 2^30 - 1; batch in 1..255 (the batch index is the
+ * voxel key's b field).  Empty scans are allowed.  d_rows fp32 [2 n_total, 5] = (b, x, y, z, t): for b = 0..batch-1
+ * the scan rows of b (t = 1, input order), then b's submap rows (t = 0): the corners sps_submap_crop_voxel returns for
+ * that scan alone, same order, bit for bit (map->ds is the lattice).  d_row_offsets int32 [batch + 1]: scan b's rows
+ * start at d_row_offsets[b]; *d_n_rows = number of rows (<= 2 n_total, so the buffer always suffices).  d_counts
+ * int32 [batch][2] = (submap voxels, unique scan voxels): sps_submap_crop_voxel's pair per scan.  Points outside the
+ * voxel-key range are left out of the crop.  d_scratch: sps_prune_batch_scratch_bytes(n_total, batch) bytes,
+ * 256-byte aligned.  No host synchronisation.  SPS_ERR_BAD_ARG: a null pointer, ld < 3, batch outside 1..255, offsets
+ * not starting at 0 or decreasing, n_total too large, misaligned scratch; SPS_ERR_CAPACITY: scratch too small. */
+size_t sps_prune_batch_scratch_bytes(int64_t n_scan_total, int batch);
+int sps_prune_batch(const sps_map* map, const float* d_scans, int64_t ld, const int64_t* h_offsets, int batch,
+                    float* d_rows, int32_t* d_row_offsets, int32_t* d_n_rows, int32_t* d_counts,
+                    void* d_scratch, size_t scratch_bytes, void* stream);
+/* sps_prune_batch -> SPSModel.forward on the rows (models.py:20-30; voxel_size is the forward's, map->ds the crop's, as
+ * in sps_infer_scan) in one call: d_scan_scores fp32 [n_total] = the scores of the scan rows, in input order (the
+ * scores of all rows go to the context's own buffer).  The forward's launches are sized by 2 n_total and the row
+ * count stays on the device, so, like a row count, 2 n_total decides the shape sort of sps_ctx_set_pattern_sort
+ * mode 1: the scores are bit-identical to sps_forward on the rows when both fall on the same side of 400 000.  A scan
+ * point outside the voxel-key range makes the context's status word report SPS_ERR_COORD_RANGE at the next
+ * sps_ctx_status.  No host synchronisation.  Errors as sps_prune_batch, plus SPS_ERR_BAD_ARG for voxel_size <= 0 and
+ * SPS_ERR_CAPACITY when 2 n_total exceeds the context's max_points. */
+int sps_infer_prune_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map, const float* d_scans, int64_t ld,
+                          const int64_t* h_offsets, int batch, float* d_rows, int32_t* d_row_offsets,
+                          int32_t* d_n_rows, int32_t* d_counts, void* d_scratch, size_t scratch_bytes,
+                          float voxel_size, float* d_scan_scores, void* stream);
+
 /* ---------------------------------------------------------------- ROS-path scan I/O (SURVEY 8f rank 3) --- */
 /* util.to_numpy (src/sps/datasets/util.py:146-153): the payload of a sensor_msgs/PointCloud2 -> fp32 [height*width,
  * nfields], every field cast to float32, fields in message order.  d_data: the message's `data` bytes on the device;

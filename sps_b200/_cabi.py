@@ -34,6 +34,7 @@ SYMBOLS = [
     "sps_pointcloud2_unpack", "sps_transform_points", "sps_pointcloud2_pack_scratch_bytes", "sps_pointcloud2_pack",
     "sps_ballmap_bytes", "sps_ballmap_build", "sps_ballmap_destroy", "sps_ball_query_scratch_bytes", "sps_submap_ball_query",
     "sps_radius_batch_scratch_bytes", "sps_radius_batch", "sps_predict_radius_batch",
+    "sps_prune_batch_scratch_bytes", "sps_prune_batch", "sps_infer_prune_batch",
 ]
 
 
@@ -140,6 +141,9 @@ def load() -> C.CDLL:
         "sps_radius_batch": (i32, [vp, vp, i64, vp, i32, vp, i64, vp, vp, vp, sz, vp]),
         "sps_predict_radius_batch": (i32, [vp, vp, vp, vp, i64, vp, i32, vp, i64, vp, vp, vp, sz, f32, f32, vp, vp, vp,
                                            vp]),
+        "sps_prune_batch_scratch_bytes": (sz, [i64, i32]),
+        "sps_prune_batch": (i32, [vp, vp, i64, vp, i32, vp, vp, vp, vp, vp, sz, vp]),
+        "sps_infer_prune_batch": (i32, [vp, vp, vp, vp, i64, vp, i32, vp, vp, vp, vp, vp, sz, f32, vp, vp]),
         "sps_profile_enable": (i32, [vp, i32]),
         "sps_profile_read": (i32, [vp, vp, vp, i32, C.POINTER(i32)]),
         "sps_ctx_pair_count": (i32, [vp, i32, i32, C.POINTER(i64), vp]),

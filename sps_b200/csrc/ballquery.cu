@@ -184,28 +184,7 @@ __global__ void k_ball_query(const float* __restrict__ scan, int64_t ld, int n_s
 // blt_dataset.py:173-182 (collate) over 209-243 (one item per scan): for b = 0..B-1 the n_b scan rows (t = 1, their
 // label), then scan b's submap rows map[idx] (t = 0, label 1), idx as sps_submap_ball_query returns it for that scan.
 // With H = the exclusive prefix of the per-point hit counts over the whole batch, scan b's rows start at
-// off[b] + H[off[b]] and scan point i's hits at off[b+1] + H[i].
-constexpr int kMaxBatch = 255;     // the batch index is the voxel key's 8-bit b field (255 is reserved)
-struct BatchOffsets { int32_t off[kMaxBatch + 1]; int batch; };   // by value: no copy, no host synchronisation
-
-__device__ __forceinline__ void load_offsets(const BatchOffsets& bo, int32_t* s_off) {
-  for (int j = threadIdx.x; j <= bo.batch; j += blockDim.x) s_off[j] = bo.off[j];
-  __syncthreads();
-}
-// scan of point i: the last b with off[b] <= i (empty scans never own a point)
-__device__ __forceinline__ int batch_of(const int32_t* s_off, int batch, int i) {
-  int lo = 0, hi = batch;
-  while (hi - lo > 1) {
-    const int mid = (lo + hi) >> 1;
-    if (s_off[mid] <= i) lo = mid; else hi = mid;
-  }
-  return lo;
-}
-// global exclusive hit prefix of point j (j == n: the total)
-__device__ __forceinline__ int hit_prefix(const int32_t* __restrict__ rank, const int32_t* __restrict__ block_sums, int n,
-                                          int total, int j) {
-  return j < n ? rank[j] + block_sums[j / kScanBlock] : total;
-}
+// off[b] + H[off[b]] and scan point i's hits at off[b+1] + H[i] (BatchOffsets, batch_of, hit_prefix: scan.cuh).
 
 // pass 1: hits of every scan point of the batch, fused with the grid-wide exclusive scan of the counts (scan.cuh)
 __global__ void __launch_bounds__(kScanBlock)

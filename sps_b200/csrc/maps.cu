@@ -1226,35 +1226,49 @@ static Scratch carve_scratch(void* base, int64_t n) {
 }
 
 // util.to_coords_features (src/sps/datasets/util.py:72-75): fp32 division by ds, then
-// `.int()` = truncation toward zero; batch and time fields are 0 in this 3-D lattice.
-__device__ inline bool trunc_key(const float* __restrict__ p, float ds, unsigned long long& key) {
+// `.int()` = truncation toward zero; the time field is 0 in this 3-D lattice, the batch field is 0 except in the
+// scratch table of a batched prune (which keeps the scans of a batch apart).
+__device__ inline bool trunc_key(const float* __restrict__ p, float ds, unsigned long long& key, int b = 0) {
   const float qx = truncf(__fdiv_rn(p[0], ds)), qy = truncf(__fdiv_rn(p[1], ds)), qz = truncf(__fdiv_rn(p[2], ds));
   const bool ok = qx >= -(float)kXBias && qx < (float)kXBias && qy >= -(float)kXBias && qy < (float)kXBias &&
                   qz >= -(float)kZBias && qz < (float)kZBias;
   if (!ok) return false;
-  key = pack_key(0, (int)qx, (int)qy, (int)qz, 0);
+  key = pack_key(b, (int)qx, (int)qy, (int)qz, 0);
   return true;
+}
+
+// point i (xyz at p, scan b) into the crop table, `first` lowered to i; out-of-range points get no slot
+__device__ __forceinline__ void insert_xyz(const float* __restrict__ p, int i, int b, float ds, Slot* tab, uint32_t mask,
+                                           uint32_t* __restrict__ slot_of, int32_t* status) {
+  unsigned long long key;
+  if (!trunc_key(p, ds, key, b)) {
+    atomicOr(status, kStatusRange);
+    if (slot_of) slot_of[i] = kInvalidSlot;
+    return;
+  }
+  const uint32_t s = table_insert(tab, mask, key);
+  atomicMin(&tab[s].first, i);
+  tab[s].val = 0;
+  if (slot_of) slot_of[i] = s;
 }
 
 __global__ void k_insert_xyz(const float* __restrict__ xyz, const int32_t* __restrict__ n_ptr, float ds, Slot* tab,
                              uint32_t* __restrict__ slot_of, int32_t* status) {
   const int n = *n_ptr;
   const uint32_t mask = table_capacity(n) - 1;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    unsigned long long key;
-    if (!trunc_key(xyz + (int64_t)i * 3, ds, key)) {
-      atomicOr(status, kStatusRange);
-      if (slot_of) slot_of[i] = kInvalidSlot;
-      continue;
-    }
-    const uint32_t s = table_insert(tab, mask, key);
-    atomicMin(&tab[s].first, i);
-    tab[s].val = 0;
-    if (slot_of) slot_of[i] = s;
-  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    insert_xyz(xyz + (int64_t)i * 3, i, 0, ds, tab, mask, slot_of, status);
 }
 
-// util.prune tail (util.py:101-112): kept voxels -> `coordinates * ds` in fp32
+// util.prune tail (util.py:101-112): a kept voxel -> `coordinates * ds` in fp32
+__device__ __forceinline__ void write_corner(unsigned long long key, float ds, float* __restrict__ o) {
+  int b, x, y, z, t;
+  unpack_key(key, b, x, y, z, t);
+  o[0] = __fmul_rn((float)x, ds);
+  o[1] = __fmul_rn((float)y, ds);
+  o[2] = __fmul_rn((float)z, ds);
+}
+
 __global__ void k_write_submap(const Slot* __restrict__ tab, const uint32_t* __restrict__ slot_of,
                                const int32_t* __restrict__ n_ptr, const int32_t* __restrict__ rank,
                                const int32_t* __restrict__ block_sums, const Slot* __restrict__ filter,
@@ -1266,11 +1280,102 @@ __global__ void k_write_submap(const Slot* __restrict__ tab, const uint32_t* __r
     const unsigned long long key = tab[s].key;
     if (table_find(filter, filter_mask, key) < 0) continue;
     const int id = rank[i] + block_sums[i / kScanBlock];
-    int b, x, y, z, t;
-    unpack_key(key, b, x, y, z, t);
-    out[(int64_t)id * 3 + 0] = __fmul_rn((float)x, ds);
-    out[(int64_t)id * 3 + 1] = __fmul_rn((float)y, ds);
-    out[(int64_t)id * 3 + 2] = __fmul_rn((float)z, ds);
+    write_corner(key, ds, out + (int64_t)id * 3);
+  }
+}
+
+// ---- batched prune: B scans concatenated -> util.infer's rows per scan, collated ----
+// Scan b's rows are its n_b scan rows [b, x, y, z, 1], then its submap rows [b, corner, 0] (sps_submap_crop_voxel of
+// scan b alone, same order).  The scratch table keys voxels by (b, trunc xyz), so scans never share a voxel and the
+// first occurrence of a voxel is its first point in scan b; the map is probed with b cleared.  With K = the exclusive
+// prefix of the "kept" flags (first occurrence and in the map) over the whole batch, scan b's rows start at
+// off[b] + K(off[b]) and the kept voxel of point i sits at off[b+1] + K(i).
+constexpr unsigned long long kKeyNoBatch = (1ull << kBShift) - 1;
+
+__global__ void k_prune_batch_insert(const float* __restrict__ scan, int64_t ld, int n, const __grid_constant__ BatchOffsets bo,
+                                     float ds, Slot* tab, uint32_t* __restrict__ slot_of, int32_t* status) {
+  __shared__ int32_t s_off[kMaxBatch + 1];
+  load_offsets(bo, s_off);
+  const uint32_t mask = table_capacity(n) - 1;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    insert_xyz(scan + (int64_t)i * ld, i, batch_of(s_off, bo.batch, i), ds, tab, mask, slot_of, status);
+}
+
+// kept flags -> grid-wide exclusive scan (scan.cuh); counts[2b+1] += unique scan voxels of scan b (counts zeroed before)
+__global__ void __launch_bounds__(kScanBlock)
+k_prune_batch_rank(const Slot* __restrict__ tab, const uint32_t* __restrict__ slot_of, int n,
+                   const __grid_constant__ BatchOffsets bo, const Slot* __restrict__ filter, uint32_t filter_mask,
+                   int32_t* __restrict__ rank, int32_t* block_sums, uint32_t* ticket, int32_t* total, int32_t* counts) {
+  __shared__ int32_t s_off[kMaxBatch + 1];
+  load_offsets(bo, s_off);
+  const int nb = max(1, (n + kScanBlock - 1) / kScanBlock);
+  const int i = blockIdx.x * kScanBlock + threadIdx.x;
+  int b = kMaxBatch + 1, first = 0;            // past-the-end lanes: a scan of their own
+  unsigned long long key = 0;
+  if (i < n) {
+    b = batch_of(s_off, bo.batch, i);
+    const uint32_t s = slot_of[i];
+    if (s != kInvalidSlot) {
+      const int4 raw = *reinterpret_cast<const int4*>(tab + s);   // key | val | first input
+      first = raw.w == i;
+      key = ((unsigned long long)(unsigned)raw.y << 32) | (unsigned)raw.x;
+    }
+  }
+  // the lanes of one scan add their first occurrences with one atomic
+  const unsigned peers = __match_any_sync(0xffffffffu, b);
+  const unsigned firsts = __ballot_sync(0xffffffffu, first) & peers;
+  if (i < n && (threadIdx.x & 31) == __ffs(peers) - 1 && firsts) atomicAdd(counts + 2 * b + 1, __popc(firsts));
+  const int kept = first && table_find(filter, filter_mask, key & kKeyNoBatch) >= 0;
+  scan_flags(kept, i, n, nb, rank, block_sums, ticket, total);
+}
+
+__device__ __forceinline__ void write_row5(float* __restrict__ rows, int64_t r, float b, float x, float y, float z, float t) {
+  float* o = rows + r * 5;
+  o[0] = b; o[1] = x; o[2] = y; o[3] = z; o[4] = t;
+}
+
+// every row at its collate position, the per-scan row offsets, the row count and counts[2b] = submap voxels of scan b
+__global__ void __launch_bounds__(256)
+k_prune_batch_write(const float* __restrict__ scan, int64_t ld, int n, const __grid_constant__ BatchOffsets bo,
+                    const Slot* __restrict__ tab, const uint32_t* __restrict__ slot_of, const int32_t* __restrict__ rank,
+                    const int32_t* __restrict__ block_sums, const int32_t* __restrict__ total_ptr, float ds,
+                    float* __restrict__ rows, int32_t* __restrict__ row_off, int32_t* __restrict__ n_rows,
+                    int32_t* __restrict__ counts) {
+  __shared__ int32_t s_off[kMaxBatch + 1];
+  load_offsets(bo, s_off);
+  const int total = *total_ptr;
+  if (blockIdx.x == 0) {
+    for (int b = threadIdx.x; b <= bo.batch; b += blockDim.x) {
+      const int k0 = hit_prefix(rank, block_sums, n, total, s_off[b]);
+      row_off[b] = s_off[b] + k0;
+      if (b < bo.batch) counts[2 * b] = hit_prefix(rank, block_sums, n, total, s_off[b + 1]) - k0;
+    }
+    if (threadIdx.x == 0) *n_rows = n + total;
+  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int b = batch_of(s_off, bo.batch, i);
+    const float* p = scan + (int64_t)i * ld;
+    const float fb = (float)b;
+    write_row5(rows, (int64_t)i + hit_prefix(rank, block_sums, n, total, s_off[b]), fb, p[0], p[1], p[2], 1.0f);
+    const int k = hit_prefix(rank, block_sums, n, total, i);
+    if (hit_prefix(rank, block_sums, n, total, i + 1) == k) continue;    // not a kept voxel
+    float c[3];
+    write_corner(tab[slot_of[i]].key, ds, c);
+    write_row5(rows, (int64_t)s_off[b + 1] + k, fb, c[0], c[1], c[2], 0.0f);
+  }
+}
+
+// fused call: the scan rows' scores in input order
+__global__ void __launch_bounds__(256)
+k_prune_batch_scores(int n, const __grid_constant__ BatchOffsets bo, const int32_t* __restrict__ rank,
+                     const int32_t* __restrict__ block_sums, const int32_t* __restrict__ total_ptr,
+                     const float* __restrict__ scores, float* __restrict__ scan_scores) {
+  __shared__ int32_t s_off[kMaxBatch + 1];
+  load_offsets(bo, s_off);
+  const int total = *total_ptr;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int b = batch_of(s_off, bo.batch, i);
+    scan_scores[i] = scores[(int64_t)i + hit_prefix(rank, block_sums, n, total, s_off[b])];
   }
 }
 
@@ -1436,4 +1541,88 @@ extern "C" int sps_infer_scan(sps_ctx* ctx, const sps_net* net, const sps_map* m
   k_assemble<<<grid_for(2 * n_scan, 256), 256, 0, st>>>(d_scan_xyz, n_scan, sub, d_counts + 0, 0.0f, rows, n_total);
   SPS_CUDA_CHECK(cudaGetLastError());
   return forward_impl(ctx, net, rows, 2 * n_scan, n_total, 5, voxel_size, d_scores, n_scan, st);
+}
+
+// ---- a batch of deployment scans: sps_submap_crop_voxel + util.infer's assembly per scan, collated ----
+namespace sps {
+
+// arguments shared by sps_prune_batch and sps_infer_prune_batch; fills `bo` and n_total
+static int check_prune_args(const sps_map* map, const float* d_scans, int64_t ld, const int64_t* h_offsets, int batch,
+                            const float* d_rows, const int32_t* d_row_offsets, const int32_t* d_n_rows,
+                            const int32_t* d_counts, const void* d_scratch, size_t scratch_bytes, BatchOffsets& bo,
+                            int64_t& n_total) {
+  if (!map || !h_offsets || !d_rows || !d_row_offsets || !d_n_rows || !d_counts || !d_scratch ||
+      ((uintptr_t)d_scratch & 255) || ld < 3 || batch < 1 || batch > kMaxBatch || h_offsets[0] != 0)
+    return SPS_ERR_BAD_ARG;
+  for (int b = 0; b < batch; ++b)
+    if (h_offsets[b + 1] < h_offsets[b]) return SPS_ERR_BAD_ARG;
+  n_total = h_offsets[batch];
+  if (n_total > 0x3fffffff || (!d_scans && n_total > 0)) return SPS_ERR_BAD_ARG;   // rows (<= 2 n_total) index as int32
+  if (scratch_bytes < carve_scratch(nullptr, n_total > 0 ? n_total : 1).bytes) return SPS_ERR_CAPACITY;
+  bo.batch = batch;
+  for (int b = 0; b <= batch; ++b) bo.off[b] = (int32_t)h_offsets[b];
+  return SPS_OK;
+}
+
+// insert -> rank -> write on the scratch carve `s`; its kept-flag ranks, chunk sums and kept total (scalars[1]) stay
+// valid for the score pass of the fused call
+static int prune_batch_launch(const sps_map* map, const float* d_scans, int64_t ld, const BatchOffsets& bo, int n,
+                              float* d_rows, int32_t* d_row_offsets, int32_t* d_n_rows, int32_t* d_counts,
+                              const Scratch& s, cudaStream_t st) {
+  const int nn = n > 0 ? n : 1;
+  SPS_CUDA_CHECK(cudaMemsetAsync(s.scalars, 0, 64 * 4, st));
+  SPS_CUDA_CHECK(cudaMemsetAsync(d_counts, 0, (size_t)bo.batch * 2 * 4, st));
+  k_level_begin<<<grid_for(s.cap, 256), 256, 0, st>>>(s.table, nullptr, n, nullptr, nullptr, 0);
+  k_prune_batch_insert<<<grid_for(nn, 256), 256, 0, st>>>(d_scans, ld, n, bo, map->ds, s.table, s.slot_of, s.scalars + 40);
+  k_prune_batch_rank<<<cdiv(nn, kScanBlock), kScanBlock, 0, st>>>(s.table, s.slot_of, n, bo, map->table, map->cap - 1,
+                                                                  s.rank, s.block_sums, (uint32_t*)(s.scalars + 32),
+                                                                  s.scalars + 1, d_counts);
+  k_prune_batch_write<<<grid_for(nn, 256), 256, 0, st>>>(d_scans, ld, n, bo, s.table, s.slot_of, s.rank, s.block_sums,
+                                                         s.scalars + 1, map->ds, d_rows, d_row_offsets, d_n_rows, d_counts);
+  SPS_CUDA_CHECK(cudaGetLastError());
+  return SPS_OK;
+}
+
+}  // namespace sps
+
+extern "C" size_t sps_prune_batch_scratch_bytes(int64_t n_scan_total, int batch) {
+  (void)batch;   // the per-scan offsets travel as kernel arguments
+  return carve_scratch(nullptr, n_scan_total > 0 ? n_scan_total : 1).bytes;
+}
+
+extern "C" int sps_prune_batch(const sps_map* map, const float* d_scans, int64_t ld, const int64_t* h_offsets, int batch,
+                               float* d_rows, int32_t* d_row_offsets, int32_t* d_n_rows, int32_t* d_counts,
+                               void* d_scratch, size_t scratch_bytes, void* stream) {
+  BatchOffsets bo;
+  int64_t n = 0;
+  const int rc = check_prune_args(map, d_scans, ld, h_offsets, batch, d_rows, d_row_offsets, d_n_rows, d_counts, d_scratch,
+                                  scratch_bytes, bo, n);
+  if (rc != SPS_OK) return rc;
+  return prune_batch_launch(map, d_scans, ld, bo, (int)n, d_rows, d_row_offsets, d_n_rows, d_counts,
+                            carve_scratch(d_scratch, n > 0 ? n : 1), (cudaStream_t)stream);
+}
+
+extern "C" int sps_infer_prune_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map, const float* d_scans, int64_t ld,
+                                     const int64_t* h_offsets, int batch, float* d_rows, int32_t* d_row_offsets,
+                                     int32_t* d_n_rows, int32_t* d_counts, void* d_scratch, size_t scratch_bytes,
+                                     float voxel_size, float* d_scan_scores, void* stream) {
+  if (!ctx || !net || !d_scan_scores || !(voxel_size > 0.f)) return SPS_ERR_BAD_ARG;
+  BatchOffsets bo;
+  int64_t n = 0;
+  int rc = check_prune_args(map, d_scans, ld, h_offsets, batch, d_rows, d_row_offsets, d_n_rows, d_counts, d_scratch,
+                            scratch_bytes, bo, n);
+  if (rc != SPS_OK) return rc;
+  if (2 * n > ctx->max_points) return SPS_ERR_CAPACITY;
+  cudaStream_t st = (cudaStream_t)stream;
+  const Scratch s = carve_scratch(d_scratch, n > 0 ? n : 1);
+  rc = prune_batch_launch(map, d_scans, ld, bo, (int)n, d_rows, d_row_offsets, d_n_rows, d_counts, s, st);
+  if (rc != SPS_OK) return rc;
+  // SPSModel.forward on the rows (models.py:20-30): the launches are sized by 2 n, the row count stays on the device;
+  // scores of every row land in the context's score buffer
+  rc = forward_impl(ctx, net, d_rows, 2 * n, d_n_rows, 5, voxel_size, ctx->scores, 2 * n, st);
+  if (rc != SPS_OK || n == 0) return rc;
+  k_prune_batch_scores<<<grid_for(n, 256), 256, 0, st>>>((int)n, bo, s.rank, s.block_sums, s.scalars + 1, ctx->scores,
+                                                        d_scan_scores);
+  SPS_CUDA_CHECK(cudaGetLastError());
+  return SPS_OK;
 }

@@ -1,4 +1,5 @@
-// Grid-wide exclusive scan of one flag per input in a single launch (block scan + last-block-done carry).
+// Grid-wide exclusive scan of one flag per input in a single launch (block scan + last-block-done carry), and the
+// helpers of the batched calls that place every scan of a batch by such a scan.
 #pragma once
 #include "ctx.h"
 
@@ -95,6 +96,29 @@ __device__ __forceinline__ int scan_flags(int flag, int i, int n, int nb, int32_
   const int excl = scan_chunk(flag, i, n, blockIdx.x, rank, block_sums);
   scan_finish(nb, nb, block_sums, ticket, count_out);
   return excl;
+}
+
+// ---- batches of B scans concatenated: scan b = inputs off[b] .. off[b+1] ----
+constexpr int kMaxBatch = 255;     // the batch index is the voxel key's 8-bit b field (255 is reserved)
+struct BatchOffsets { int32_t off[kMaxBatch + 1]; int batch; };   // by value: no copy, no host synchronisation
+
+__device__ __forceinline__ void load_offsets(const BatchOffsets& bo, int32_t* s_off) {
+  for (int j = threadIdx.x; j <= bo.batch; j += blockDim.x) s_off[j] = bo.off[j];
+  __syncthreads();
+}
+// scan of point i: the last b with off[b] <= i (empty scans never own a point)
+__device__ __forceinline__ int batch_of(const int32_t* s_off, int batch, int i) {
+  int lo = 0, hi = batch;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if (s_off[mid] <= i) lo = mid; else hi = mid;
+  }
+  return lo;
+}
+// global exclusive prefix of the scanned flags (or counts) at input j (j == n: the total)
+__device__ __forceinline__ int hit_prefix(const int32_t* __restrict__ rank, const int32_t* __restrict__ block_sums, int n,
+                                          int total, int j) {
+  return j < n ? rank[j] + block_sums[j / kScanBlock] : total;
 }
 
 

@@ -25,11 +25,12 @@ SCAN_TIMESTAMP, MAP_TIMESTAMP = 1.0, 0.0     # src/sps/datasets/util.py:20-21
 MAX_BATCH = 255                               # scans per batch: the batch index is the voxel key's 8-bit b field
 
 
-def batch_parts(scans, offsets=None):
-    """A batch of scans as the library takes it: ``scans`` is a list of per-scan fp32 ``[n_b, >=4]`` tensors (x, y, z,
-    label, in the map frame), or one ``[sum n_b, >=4]`` tensor with ``offsets`` (``B + 1`` ints, scan b = rows
-    ``offsets[b]:offsets[b+1]``).  Returns ``(parts, offsets, ld)``: ``parts`` = [(contiguous fp32 tensor, first row)],
-    ``offsets`` a list of B + 1 ints, ``ld`` the common row width."""
+def batch_parts(scans, offsets=None, min_width=4):
+    """A batch of scans as the library takes it: ``scans`` is a list of per-scan fp32 ``[n_b, >=min_width]`` tensors
+    (x, y, z, label, in the map frame; the deployment path has no label and passes ``min_width=3``), or one
+    ``[sum n_b, >=min_width]`` tensor with ``offsets`` (``B + 1`` ints, scan b = rows ``offsets[b]:offsets[b+1]``).
+    Returns ``(parts, offsets, ld)``: ``parts`` = [(contiguous fp32 tensor, first row)], ``offsets`` a list of B + 1
+    ints, ``ld`` the common row width."""
     if isinstance(scans, torch.Tensor):
         if offsets is None:
             raise ValueError("one scan tensor needs the per-scan offsets")
@@ -50,10 +51,22 @@ def batch_parts(scans, offsets=None):
     if offsets[0] != 0 or any(b < a for a, b in zip(offsets, offsets[1:])):
         raise ValueError("offsets must start at 0 and never decrease")
     widths = {t.shape[1] for t in scans if t.dim() == 2}
-    if len(widths) != 1 or any(t.dim() != 2 for t in scans) or min(widths) < 4:
-        raise ValueError("scans must be 2-D with one common width >= 4 (x, y, z, label)")
+    if len(widths) != 1 or any(t.dim() != 2 for t in scans) or min(widths) < min_width:
+        cols = "x, y, z, label" if min_width >= 4 else "x, y, z"
+        raise ValueError(f"scans must be 2-D with one common width >= {min_width} ({cols})")
     parts = [(t.contiguous().float(), s) for t, s in zip(scans, starts)]
     return parts, offsets, widths.pop()
+
+
+def device_scans(parts, n, ld, device):
+    """The scans of :func:`batch_parts` as one device tensor ``[max(n, 1), ld]``: the single part itself when it already
+    lives on ``device``, else a new tensor the parts are copied into (on the current stream)."""
+    if len(parts) == 1 and parts[0][0].device == device:
+        return parts[0][0]
+    src = torch.empty((max(n, 1), ld), dtype=torch.float32, device=device)
+    for t, start in parts:
+        src[start:start + t.shape[0]].copy_(t)
+    return src
 
 
 class RadiusSubmap:
@@ -124,12 +137,7 @@ class RadiusSubmap:
         parts, offs, ld = batch_parts(scans, offsets)
         dev = self.map_xyz.device
         n, batch = offs[-1], len(offs) - 1
-        if len(parts) == 1 and parts[0][0].device == dev:
-            src = parts[0][0]
-        else:
-            src = torch.empty((max(n, 1), ld), dtype=torch.float32, device=dev)
-            for t, start in parts:
-                src[start:start + t.shape[0]].copy_(t)
+        src = device_scans(parts, n, ld, dev)
         nbytes = self.lib.sps_radius_batch_scratch_bytes(n, batch)
         scratch = torch.empty(nbytes + 256, dtype=torch.uint8, device=dev)
         sbase = (scratch.data_ptr() + 255) & ~255

@@ -315,6 +315,30 @@ class MapHash:
         return out[:m], nuniq
 
     @_on_device
+    def prune_batch(self, scans, offsets=None):
+        """:meth:`crop_voxel` + ``util.infer``'s assembly for every scan of a batch, collated, in the library
+        (``sps_prune_batch``).  ``scans``: a list of per-scan fp32 ``[n_b, >=3]`` tensors (x, y, z in the map frame;
+        further columns are ignored) or one ``[sum n_b, >=3]`` tensor plus ``offsets`` (``B + 1`` ints), on the device
+        or on the host.  Returns device tensors ``(rows [R, 5], row_offsets int32 [B + 1], counts int32 [B, 2])``: per
+        scan its rows ``[b, x, y, z, 1]``, then its submap rows ``[b, corner, 0]`` (bit-identical to stacking the
+        per-scan rows built from ``crop_voxel``), and ``crop_voxel``'s ``(len(submap), n_unique_scan_voxels)``.  One
+        host synchronisation (the row count sizes the result)."""
+        from .datasets import batch_parts, device_scans
+        parts, offs, ld = batch_parts(scans, offsets, min_width=3)
+        n, batch = offs[-1], len(offs) - 1
+        src = device_scans(parts, n, ld, self.device)
+        nbytes = self.lib.sps_prune_batch_scratch_bytes(n, batch)
+        scratch = self._scratch_for(nbytes)
+        rows = torch.empty((max(2 * n, 1), 5), dtype=torch.float32, device=self.device)
+        row_offsets = torch.empty(batch + 1, dtype=torch.int32, device=self.device)
+        n_rows = torch.empty(1, dtype=torch.int32, device=self.device)
+        counts = torch.empty((batch, 2), dtype=torch.int32, device=self.device)
+        h_off = (C.c_int64 * (batch + 1))(*offs)
+        check(self.lib.sps_prune_batch(self.handle, _ptr(src), ld, h_off, batch, _ptr(rows), _ptr(row_offsets), _ptr(n_rows),
+                                       _ptr(counts), _ptr(scratch), nbytes, _stream()), "sps_prune_batch")
+        return rows[:int(n_rows.item())], row_offsets, counts
+
+    @_on_device
     def crop_radius(self, center, radius: float) -> torch.Tensor:
         """MapMOS-style radius crop: indices (int32, map order) of map points within ``radius``."""
         n = self.map_xyz.shape[0]

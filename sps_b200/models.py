@@ -133,16 +133,17 @@ class CustomMinkUNet(nn.Module):
 
 
 class _Pending:
-    """Handle of an in-flight ``SPSModel.forward_async`` call."""
+    """Handle of an in-flight ``SPSModel.forward_async`` or ``SPSModel.infer_scans_async`` call."""
 
     def __init__(self, event, out, engine, device_scores=None):
         self._event, self._out, self._engine = event, out, engine
         # the scores on the device (valid once the call is done; the lane reuses the buffer `lanes` calls later)
         self.device_scores = device_scores if device_scores is not None else out
 
-    def result(self, check: bool = True) -> torch.Tensor:
-        """Wait for the call and return its scores.  ``check`` (default) also reads the engine's sticky status word,
-        so a coordinate outside the voxel-key range raises here instead of leaving NaN scores behind."""
+    def result(self, check: bool = True):
+        """Wait for the call and return its results (forward_async: the scores).  ``check`` (default) also reads the
+        engine's sticky status word, so a coordinate outside the voxel-key range raises here instead of leaving NaN
+        scores behind."""
         self._event.synchronize()
         if check:
             self._engine.status()
@@ -168,6 +169,18 @@ class _PendingRadius:
                     raise
                 return self._retry(int(self._n_rows[0])).result(check)
         return self._out
+
+
+def _lane_buffers(buf, device):
+    """``grow(name, shape, dtype, pinned=False)``: the lane buffer ``buf[name]``, (re)allocated when it is missing or
+    has fewer than ``shape[0]`` rows -- on ``device``, or in pinned host memory."""
+    def grow(name, shape, dtype, pinned=False):
+        t = buf.get(name)
+        if t is None or t.shape[0] < shape[0]:
+            t = torch.empty(shape, dtype=dtype, device="cpu" if pinned else device)
+            buf[name] = t.pin_memory() if pinned else t
+        return buf[name]
+    return grow
 
 
 class SPSModel(nn.Module):
@@ -310,7 +323,7 @@ class SPSModel(nn.Module):
                               "d_out": [torch.empty(cap, dtype=torch.float32, device=device) for _ in range(self.lanes)],
                               "h_out": [torch.empty(cap, dtype=torch.float32).pin_memory() for _ in range(self.lanes)],
                               "busy": [None] * self.lanes, "graphs": [dict() for _ in range(self.lanes)],
-                              "radius": [dict() for _ in range(self.lanes)]}
+                              "radius": [dict() for _ in range(self.lanes)], "prune": [dict() for _ in range(self.lanes)]}
         return p, net
 
     def _next_lane(self, p):
@@ -355,14 +368,7 @@ class SPSModel(nn.Module):
         on_device = all(t.is_cuda for t, _ in parts)
         buf = p["radius"][slot]
         lib = lane_engine.lib
-
-        def grow(name, shape, dtype, pinned=False):
-            t = buf.get(name)
-            if t is None or t.shape[0] < shape[0]:
-                t = torch.empty(shape, dtype=dtype, device="cpu" if pinned else device)
-                buf[name] = t.pin_memory() if pinned else t
-            return buf[name]
-
+        grow = _lane_buffers(buf, device)
         nbytes = lib.sps_radius_batch_scratch_bytes(n, batch)
         rows = grow("rows", (cap, 6), torch.float32)
         scratch = grow("scratch", (nbytes,), torch.uint8)    # the caching allocator hands out 512-byte aligned blocks
@@ -372,18 +378,7 @@ class SPSModel(nn.Module):
         counts = grow("counts", (MAX_BATCH, 4), torch.int64)
         sums = grow("sums", (MAX_BATCH, 5), torch.float64)
         compute.wait_stream(torch.cuda.current_stream(device))
-        if len(parts) == 1 and on_device and parts[0][0].device == device:
-            src = parts[0][0]
-        else:
-            src = grow(("scans", ld), (max(n, 1), ld), torch.float32)
-            copy = compute if on_device else p["copy"]
-            with torch.cuda.stream(copy):
-                for t, start in parts:
-                    src[start:start + t.shape[0]].copy_(t, non_blocking=True)
-                ready = torch.cuda.Event()
-                ready.record(copy)
-            compute.wait_event(ready)
-        buf["keep"] = (parts, src)                          # alive until the lane's next call
+        src = self._lane_scans(p, buf, grow, parts, n, ld, on_device, compute, device)
         h_off = (C.c_int64 * (batch + 1))(*offs)
         with torch.cuda.device(device), torch.cuda.stream(compute):
             check(lib.sps_predict_radius_batch(lane_engine.handle, net.handle, submap.handle, _ptr(src), ld, h_off, batch,
@@ -406,6 +401,82 @@ class SPSModel(nn.Module):
         def retry(true_rows):
             return self._predict_radius(parts, offs, ld, submap, eps, true_rows)
         return _PendingRadius(done, out, lane_engine, h_rows, retry)
+
+    @staticmethod
+    def _lane_scans(p, buf, grow, parts, n, ld, on_device, compute, device):
+        """The scans of a batched call on the device, ready on the lane's stream ``compute``: a single device part is
+        read in place; otherwise the parts are copied into the lane's staging buffer, host parts on the copy stream (the
+        copies of call k+1 overlap the kernels of call k).  The sources stay alive until the lane's next call."""
+        if len(parts) == 1 and on_device and parts[0][0].device == device:
+            src = parts[0][0]
+        else:
+            src = grow(("scans", ld), (max(n, 1), ld), torch.float32)
+            copy = compute if on_device else p["copy"]
+            with torch.cuda.stream(copy):
+                for t, start in parts:
+                    src[start:start + t.shape[0]].copy_(t, non_blocking=True)
+                ready = torch.cuda.Event()
+                ready.record(copy)
+            compute.wait_event(ready)
+        buf["keep"] = (parts, src)
+        return src
+
+    def infer_scans_async(self, scans, map_hash, offsets=None):
+        """The ROS node's per-scan loop body (``sps_node.py:111-120``: ``util.prune`` against the base map, then
+        ``util.infer``) for a whole batch of scans in one asynchronous library call (``sps_infer_prune_batch``): every
+        scan's voxel-pruned submap from ``map_hash`` (a :class:`sps_b200.engine.MapHash`; its ``ds`` is the crop
+        lattice, this model's voxel size the forward's), the collated rows, one ``forward`` on them.  ``scans``: a list
+        of per-scan fp32 ``[n_b, >=3]`` tensors (x, y, z in the map frame; further columns are ignored) or one
+        ``[sum n_b, >=3]`` tensor plus ``offsets`` (``B + 1`` ints); 1..255 scans, empty ones allowed.
+
+        Returns a handle whose ``result()`` gives ``(scan_scores [sum n_b], counts int32 [B, 2])``: the scores of the
+        scan points in input order (those of ``util.infer`` on each scan's rows) and per scan ``MapHash.crop_voxel``'s
+        ``(len(submap), n_unique_scan_voxels)``; it raises :class:`SpsError` when a point lay outside the voxel-key
+        range.  Device scans are read in place and the results stay on the device; host (preferably pinned) scans go
+        to the device on the copy stream and the results come back to pinned host memory.  Either way the buffers
+        belong to one of the model's lanes, whose contexts hold ``2 * sum n_b`` rows: the call ``lanes`` calls later
+        reuses them.  The forward is sized by ``2 * sum n_b`` rows, which, like a row count, decides the default shape
+        sort (``sps_ctx_set_pattern_sort`` mode 1)."""
+        if self.training:
+            raise RuntimeError("sps_b200 is inference-only (call .eval()); training is out of scope")
+        parts, offs, ld = batch_parts(scans, offsets, min_width=3)
+        device = next(self.MinkUNet.parameters()).device
+        if device.type != "cuda":
+            raise RuntimeError("move the model to a CUDA device first: sps_b200 has no CPU path")
+        if norm_device(map_hash.device) != norm_device(device):
+            raise RuntimeError("the map hash must live on the model's device")
+        n, batch = offs[-1], len(offs) - 1
+        p, net = self._lanes(max(2 * n, 1), None, device)
+        slot = self._next_lane(p)
+        lane_engine, compute = p["engine"][slot], p["stream"][slot]
+        on_device = all(t.is_cuda for t, _ in parts)
+        buf = p["prune"][slot]
+        lib = lane_engine.lib
+        grow = _lane_buffers(buf, device)
+        nbytes = lib.sps_prune_batch_scratch_bytes(n, batch)
+        rows = grow("rows", (max(2 * n, 1), 5), torch.float32)
+        scratch = grow("scratch", (nbytes,), torch.uint8)    # the caching allocator hands out 512-byte aligned blocks
+        row_offsets = grow("row_offsets", (MAX_BATCH + 1,), torch.int32)
+        n_rows = grow("n_rows", (1,), torch.int32)
+        scores = grow("scores", (max(n, 1),), torch.float32)
+        counts = grow("counts", (MAX_BATCH, 2), torch.int32)
+        compute.wait_stream(torch.cuda.current_stream(device))
+        src = self._lane_scans(p, buf, grow, parts, n, ld, on_device, compute, device)
+        h_off = (C.c_int64 * (batch + 1))(*offs)
+        with torch.cuda.device(device), torch.cuda.stream(compute):
+            check(lib.sps_infer_prune_batch(lane_engine.handle, net.handle, map_hash.handle, _ptr(src), ld, h_off, batch,
+                                            _ptr(rows), _ptr(row_offsets), _ptr(n_rows), _ptr(counts), _ptr(scratch), nbytes,
+                                            self.voxel_size, _ptr(scores), _stream(device)), "sps_infer_prune_batch")
+            out = (scores[:n], counts[:batch])
+            if not on_device:
+                h = (grow("h_scores", (max(n, 1),), torch.float32, True), grow("h_counts", (MAX_BATCH, 2), torch.int32, True))
+                out = (h[0][:n], h[1][:batch])
+                for dst, s in zip(out, (scores[:n], counts[:batch])):
+                    dst.copy_(s, non_blocking=True)
+            done = torch.cuda.Event()
+            done.record(compute)
+        p["busy"][slot] = done
+        return _Pending(done, out, lane_engine)
 
     def _lane_forward(self, p, slot, lane_engine, net, src, d_out, compute):
         """One forward on a lane's stream (current), eagerly or as a CUDA-graph replay.  Every size that only exists on
