@@ -280,6 +280,34 @@ int sps_infer_prune_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map, 
                           const int64_t* h_offsets, int batch, float* d_rows, int32_t* d_row_offsets,
                           int32_t* d_n_rows, int32_t* d_counts, void* d_scratch, size_t scratch_bytes,
                           float voxel_size, float* d_scan_scores, void* stream);
+/* The ROS node's callback (sps_node.py:88-176) for a batch of SENSOR-frame scans in one call.  Per scan b: its points
+ * moved into the map frame with its pose, sps_infer_prune_batch on them, the node's metrics and the published rows.
+ * d_scans fp32 [n_total, ld >= 4] = sensor-frame x, y, z and column 3 per point (further columns are ignored);
+ * h_offsets and batch as sps_prune_batch.  Column 3 is the `intensity` field the node publishes and also the label
+ * its metrics are computed against (SURVEY §3.2, sps_node.py:123-134; taken from the survey, the reference source was
+ * not at hand to check it).  d_poses (DEVICE) float64 [batch][16]: each scan's row-major 4x4 matrix
+ * (util.to_tr_matrix); the transform is sps_transform_points' arithmetic, so every transformed scan is bit-identical
+ * to sps_transform_points on that scan alone.  Outputs:
+ *   d_rows, d_row_offsets, d_n_rows, d_counts: sps_prune_batch on the map-frame points (the rows hold them);
+ *   d_scan_scores fp32 [n_total]: the scan rows' scores in input order, bit-identical to sps_infer_prune_batch on the
+ *     map-frame scans;
+ *   d_metric_counts int64 [batch][4], d_metric_sums double [batch][5]: per-scan partials in sps_confusion_counts'
+ *     layout, pred = score < eps, gt = column 3 < eps (empty scans: zeros);
+ *   d_kept fp32 [n_total, 4] (16-byte aligned): sensor-frame x, y, z, column 3 of every point whose score is <= eps
+ *     (NaN scores are dropped), scan after scan in input order: sps_pointcloud2_pack per scan, laid end to end;
+ *   d_kept_offsets int32 [batch + 1]: scan b's published rows are d_kept[d_kept_offsets[b] .. d_kept_offsets[b+1]).
+ * d_scratch: sps_filter_scans_batch_scratch_bytes(n_total, batch) bytes, 256-byte aligned.  A map-frame point
+ * outside the voxel-key range makes the context's status word report SPS_ERR_COORD_RANGE at the next
+ * sps_ctx_status.  No host synchronisation.  Errors as sps_infer_prune_batch, plus SPS_ERR_BAD_ARG for ld < 4, a null
+ * d_poses, d_kept, d_kept_offsets or metric buffer, a d_kept that is not 16-byte aligned and a NaN eps. */
+size_t sps_filter_scans_batch_scratch_bytes(int64_t n_scan_total, int batch);
+int sps_filter_scans_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map,
+                           const float* d_scans, int64_t ld, const int64_t* h_offsets, int batch,
+                           const double* d_poses, float eps, float voxel_size,
+                           float* d_rows, int32_t* d_row_offsets, int32_t* d_n_rows, int32_t* d_counts,
+                           float* d_scan_scores, int64_t* d_metric_counts, double* d_metric_sums,
+                           float* d_kept, int32_t* d_kept_offsets,
+                           void* d_scratch, size_t scratch_bytes, void* stream);
 
 /* ---------------------------------------------------------------- ROS-path scan I/O (SURVEY 8f rank 3) --- */
 /* util.to_numpy (src/sps/datasets/util.py:146-153): the payload of a sensor_msgs/PointCloud2 -> fp32 [height*width,

@@ -10,7 +10,9 @@
 #include <limits.h>
 #include <utility>
 #include "ctx.h"
+#include "partials.cuh"
 #include "profile.h"
+#include "rosio.cuh"
 #include "scan.cuh"
 
 namespace sps {
@@ -1623,6 +1625,108 @@ extern "C" int sps_infer_prune_batch(sps_ctx* ctx, const sps_net* net, const sps
   if (rc != SPS_OK || n == 0) return rc;
   k_prune_batch_scores<<<grid_for(n, 256), 256, 0, st>>>((int)n, bo, s.rank, s.block_sums, s.scalars + 1, ctx->scores,
                                                         d_scan_scores);
+  SPS_CUDA_CHECK(cudaGetLastError());
+  return SPS_OK;
+}
+
+// ---- a batch of sensor-frame deployment scans: the ROS node's callback (sps_node.py:88-176) per scan, collated ----
+// Per scan: the pose transform into the map frame (util.transform_point_cloud), util.prune + util.infer (the launches of
+// sps_infer_prune_batch on the transformed scans), the node's metrics against column 3 and the published rows (score
+// <= eps, sensor frame).  The partials are k_radius_partials (partials.cuh) on the prune layout, the published rows one
+// compaction of the whole batch (k_filter_rank / k_filter_write, rosio.cuh): the scans are concatenated in order, so it
+// is the per-scan compactions laid end to end.
+namespace sps {
+
+// point i -> the map frame with its scan's pose (transform_point, rosio.cuh); a run of threads reads the same 128 bytes
+__global__ void __launch_bounds__(256)
+k_transform_batch(const float* __restrict__ scan, int64_t ld, int n, const __grid_constant__ BatchOffsets bo,
+                  const double* __restrict__ poses, float* __restrict__ xyz) {
+  __shared__ int32_t s_off[kMaxBatch + 1];
+  load_offsets(bo, s_off);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    transform_point(scan, ld, i, poses + 16 * batch_of(s_off, bo.batch, i), xyz);
+}
+
+// kept_off[b] = published rows of the scans before b: the filter's exclusive prefix at b's first point
+__global__ void k_kept_offsets(int n, const __grid_constant__ BatchOffsets bo, const int32_t* __restrict__ rank,
+                               const int32_t* __restrict__ block_sums, const int32_t* __restrict__ total_ptr,
+                               int32_t* __restrict__ kept_off) {
+  const int total = *total_ptr;
+  for (int b = threadIdx.x; b <= bo.batch; b += blockDim.x) kept_off[b] = hit_prefix(rank, block_sums, n, total, bo.off[b]);
+}
+
+// scratch of the filter call: map-frame xyz [n, 3] | the prune carve | the filter's ranks, chunk sums, ticket line
+// (ticket, kept total)
+struct FilterCarve {
+  float* xyz; Scratch prune; int32_t* rank; int32_t* block_sums; uint32_t* ticket; int32_t* total; size_t bytes;
+};
+static FilterCarve carve_filter(void* base, int64_t n) {
+  FilterCarve c;
+  char* p = (char*)base;
+  size_t off = 0;
+  auto take = [&](size_t b) { off = (off + 255) & ~size_t(255); char* r = p ? p + off : nullptr; off += b; return r; };
+  c.xyz = (float*)take((size_t)n * 3 * 4);
+  c.prune = carve_scratch(take(carve_scratch(nullptr, n).bytes), n);
+  c.rank = (int32_t*)take((size_t)n * 4);
+  c.block_sums = (int32_t*)take((size_t)(n / kScanBlock + 2) * 4);
+  c.ticket = (uint32_t*)take(256);
+  c.total = (int32_t*)(c.ticket + 1);
+  c.bytes = (off + 255) & ~size_t(255);
+  return c;
+}
+
+}  // namespace sps
+
+extern "C" size_t sps_filter_scans_batch_scratch_bytes(int64_t n_scan_total, int batch) {
+  (void)batch;   // the per-scan offsets travel as kernel arguments
+  return carve_filter(nullptr, n_scan_total > 0 ? n_scan_total : 1).bytes;
+}
+
+extern "C" int sps_filter_scans_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map, const float* d_scans, int64_t ld,
+                                      const int64_t* h_offsets, int batch, const double* d_poses, float eps,
+                                      float voxel_size, float* d_rows, int32_t* d_row_offsets, int32_t* d_n_rows,
+                                      int32_t* d_counts, float* d_scan_scores, int64_t* d_metric_counts,
+                                      double* d_metric_sums, float* d_kept, int32_t* d_kept_offsets, void* d_scratch,
+                                      size_t scratch_bytes, void* stream) {
+  if (!ctx || !net || !d_scan_scores || !d_poses || !d_metric_counts || !d_metric_sums || !d_kept || !d_kept_offsets ||
+      ((uintptr_t)d_kept & 15) || ld < 4 || eps != eps || !(voxel_size > 0.f))
+    return SPS_ERR_BAD_ARG;
+  BatchOffsets bo;
+  int64_t n = 0;
+  int rc = check_prune_args(map, d_scans, ld, h_offsets, batch, d_rows, d_row_offsets, d_n_rows, d_counts, d_scratch,
+                            scratch_bytes, bo, n);
+  if (rc != SPS_OK) return rc;
+  const FilterCarve c = carve_filter(d_scratch, n > 0 ? n : 1);
+  if (scratch_bytes < c.bytes || 2 * n > ctx->max_points) return SPS_ERR_CAPACITY;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (n > 0) {
+    k_transform_batch<<<grid_for(n, 256), 256, 0, st>>>(d_scans, ld, (int)n, bo, d_poses, c.xyz);
+    SPS_CUDA_CHECK(cudaGetLastError());
+  }
+  // sps_infer_prune_batch on the map-frame scans: the rows, then the forward on them (scores in the context's buffer)
+  rc = prune_batch_launch(map, c.xyz, 3, bo, (int)n, d_rows, d_row_offsets, d_n_rows, d_counts, c.prune, st);
+  if (rc != SPS_OK) return rc;
+  rc = forward_impl(ctx, net, d_rows, 2 * n, d_n_rows, 5, voxel_size, ctx->scores, 2 * n, st);
+  if (rc != SPS_OK) return rc;
+  SPS_CUDA_CHECK(cudaMemsetAsync(d_metric_counts, 0, (size_t)batch * 4 * sizeof(int64_t), st));
+  SPS_CUDA_CHECK(cudaMemsetAsync(d_metric_sums, 0, (size_t)batch * 5 * sizeof(double), st));
+  if (n == 0) {
+    SPS_CUDA_CHECK(cudaMemsetAsync(d_kept_offsets, 0, (size_t)(batch + 1) * 4, st));
+    return SPS_OK;
+  }
+  // scan point i's row is i + K(off[b]) (the prune's kept-flag prefix); every row is scored (n_rows == n_fwd); the
+  // labels are column 3 of the sensor-frame input
+  const int per_block = 256 * kPartialsSpan;
+  k_radius_partials<<<cdiv(n, per_block), 256, 0, st>>>(d_scans, ld, (int)n, bo, c.prune.rank, c.prune.block_sums,
+                                                       c.prune.scalars + 1, d_n_rows, d_n_rows, ctx->scores, eps,
+                                                       d_scan_scores, reinterpret_cast<unsigned long long*>(d_metric_counts),
+                                                       d_metric_sums);
+  // the published rows: sps_pointcloud2_pack over the whole batch, plus where each scan's rows start
+  SPS_CUDA_CHECK(cudaMemsetAsync(c.ticket, 0, 256, st));
+  k_filter_rank<<<cdiv(n, kScanBlock), kScanBlock, 0, st>>>(d_scan_scores, (int)n, eps, c.rank, c.block_sums, c.ticket,
+                                                            c.total);
+  k_filter_write<<<grid_for(n, 256, 148 * 16), 256, 0, st>>>(d_scans, ld, n, d_scan_scores, eps, c.rank, c.block_sums, d_kept);
+  k_kept_offsets<<<1, 256, 0, st>>>((int)n, bo, c.rank, c.block_sums, c.total, d_kept_offsets);
   SPS_CUDA_CHECK(cudaGetLastError());
   return SPS_OK;
 }

@@ -13,6 +13,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+from typing import NamedTuple
 
 import numpy as np
 import torch
@@ -171,6 +172,29 @@ class _PendingRadius:
         return self._out
 
 
+class FilteredScans(NamedTuple):
+    """Results of ``SPSModel.filter_scans_async`` for a batch of B scans of n_total points."""
+    scan_scores: torch.Tensor    # fp32 [n_total]: the scan points' scores, in input order
+    kept: torch.Tensor           # fp32 [K, 4]: the published rows (sensor-frame x, y, z, column 3), scan after scan
+    kept_offsets: torch.Tensor   # int32 [B + 1]: scan b's published rows are kept[kept_offsets[b]:kept_offsets[b+1]]
+    counts: torch.Tensor         # int32 [B, 2]: MapHash.crop_voxel's (len(submap), n_unique_scan_voxels) per scan
+    metric_counts: torch.Tensor  # int64 [B, 4]: per-scan confusion counts (parallel.device_partials' layout)
+    metric_sums: torch.Tensor    # float64 [B, 5]: per-scan sums (parallel.device_partials' layout)
+
+
+class _PendingFilter(_Pending):
+    """Handle of an in-flight ``SPSModel.filter_scans_async`` call."""
+
+    def __init__(self, event, out, engine, kept_end):
+        super().__init__(event, out, engine)
+        self._kept_end = kept_end     # pinned host int32 [1]: K, once the call is done
+
+    def result(self, check: bool = True) -> FilteredScans:
+        """Wait for the call and return its :class:`FilteredScans` (``check``: as ``_Pending.result``)."""
+        out = super().result(check)
+        return out._replace(kept=out.kept[:int(self._kept_end[0])])
+
+
 def _lane_buffers(buf, device):
     """``grow(name, shape, dtype, pinned=False)``: the lane buffer ``buf[name]``, (re)allocated when it is missing or
     has fewer than ``shape[0]`` rows -- on ``device``, or in pinned host memory."""
@@ -323,7 +347,8 @@ class SPSModel(nn.Module):
                               "d_out": [torch.empty(cap, dtype=torch.float32, device=device) for _ in range(self.lanes)],
                               "h_out": [torch.empty(cap, dtype=torch.float32).pin_memory() for _ in range(self.lanes)],
                               "busy": [None] * self.lanes, "graphs": [dict() for _ in range(self.lanes)],
-                              "radius": [dict() for _ in range(self.lanes)], "prune": [dict() for _ in range(self.lanes)]}
+                              "radius": [dict() for _ in range(self.lanes)], "prune": [dict() for _ in range(self.lanes)],
+                              "filter": [dict() for _ in range(self.lanes)]}
         return p, net
 
     def _next_lane(self, p):
@@ -477,6 +502,93 @@ class SPSModel(nn.Module):
             done.record(compute)
         p["busy"][slot] = done
         return _Pending(done, out, lane_engine)
+
+    def filter_scans_async(self, scans, poses, map_hash, eps: float, offsets=None):
+        """The ROS node's whole callback (``sps_node.py:88-176``) for a batch of sensor-frame scans in one asynchronous
+        library call (``sps_filter_scans_batch``): every scan moved into the map frame with its pose
+        (``util.transform_point_cloud``), ``infer_scans_async`` on the moved scans, the node's metrics against the
+        scan's column 3 (``pred = score < eps``, ``gt = label < eps``) and the rows the node publishes
+        (``util.filter_scan``: sensor-frame x, y, z, column 3 of the points whose score is ``<= eps``).  ``scans``: a
+        list of per-scan fp32 ``[n_b, >=4]`` tensors (x, y, z, intensity in the sensor frame; the intensity is also
+        the label) or one ``[sum n_b, >=4]`` tensor plus ``offsets``; ``poses``: float64 ``[B, 4, 4]`` (numpy array or
+        tensor, on the host or the device), scan b's row-major matrix (``util.to_tr_matrix``).
+
+        Returns a handle whose ``result()`` gives a :class:`FilteredScans`; it raises :class:`SpsError` when a
+        map-frame point lay outside the voxel-key range.  ``parallel.per_scan_metrics(metric_counts, metric_sums)``
+        gives the node's per-scan values, ``util.to_rosmsg(kept[o[b]:o[b+1]], header)`` scan b's message.  Device
+        scans give device results; host (preferably pinned) scans go to the device on the copy stream and the results
+        come back to pinned host memory (the whole ``[sum n_b, 4]`` buffer of published rows, which ``result()``
+        slices).  Host poses go through a pinned buffer of the lane on the copy stream.  Either way the buffers belong
+        to one of the model's lanes: the call ``lanes`` calls later reuses them."""
+        if self.training:
+            raise RuntimeError("sps_b200 is inference-only (call .eval()); training is out of scope")
+        parts, offs, ld = batch_parts(scans, offsets, min_width=4)
+        n, batch = offs[-1], len(offs) - 1
+        poses = poses if isinstance(poses, torch.Tensor) else torch.as_tensor(np.asarray(poses))
+        if poses.dtype != torch.float64 or tuple(poses.shape) != (batch, 4, 4):
+            raise ValueError(f"poses must be float64 [{batch}, 4, 4] (one matrix per scan), got {poses.dtype} "
+                             f"{tuple(poses.shape)}")
+        device = next(self.MinkUNet.parameters()).device
+        if device.type != "cuda":
+            raise RuntimeError("move the model to a CUDA device first: sps_b200 has no CPU path")
+        if norm_device(map_hash.device) != norm_device(device):
+            raise RuntimeError("the map hash must live on the model's device")
+        if poses.is_cuda and poses.device != device:
+            raise RuntimeError("device poses must live on the model's device")
+        p, net = self._lanes(max(2 * n, 1), None, device)
+        slot = self._next_lane(p)
+        lane_engine, compute = p["engine"][slot], p["stream"][slot]
+        on_device = all(t.is_cuda for t, _ in parts)
+        buf = p["filter"][slot]
+        lib = lane_engine.lib
+        grow = _lane_buffers(buf, device)
+        nbytes = lib.sps_filter_scans_batch_scratch_bytes(n, batch)
+        rows = grow("rows", (max(2 * n, 1), 5), torch.float32)
+        scratch = grow("scratch", (nbytes,), torch.uint8)    # the caching allocator hands out 512-byte aligned blocks
+        row_offsets = grow("row_offsets", (MAX_BATCH + 1,), torch.int32)
+        n_rows = grow("n_rows", (1,), torch.int32)
+        scores = grow("scores", (max(n, 1),), torch.float32)
+        counts = grow("counts", (MAX_BATCH, 2), torch.int32)
+        metric_counts = grow("metric_counts", (MAX_BATCH, 4), torch.int64)
+        metric_sums = grow("metric_sums", (MAX_BATCH, 5), torch.float64)
+        kept = grow("kept", (max(n, 1), 4), torch.float32)
+        kept_offsets = grow("kept_offsets", (MAX_BATCH + 1,), torch.int32)
+        if poses.is_cuda:
+            d_poses = poses.contiguous()                   # (on the current stream, which the lane's stream waits for)
+            buf["keep_poses"] = d_poses                     # alive until the lane's next call
+        compute.wait_stream(torch.cuda.current_stream(device))
+        src = self._lane_scans(p, buf, grow, parts, n, ld, on_device, compute, device)
+        if not poses.is_cuda:
+            h_poses = grow("h_poses", (MAX_BATCH, 4, 4), torch.float64, True)
+            h_poses[:batch].copy_(poses)
+            d_poses = grow("poses", (MAX_BATCH, 4, 4), torch.float64)
+            with torch.cuda.stream(p["copy"]):
+                d_poses[:batch].copy_(h_poses[:batch], non_blocking=True)
+                ready = torch.cuda.Event()
+                ready.record(p["copy"])
+            compute.wait_event(ready)
+        h_off = (C.c_int64 * (batch + 1))(*offs)
+        with torch.cuda.device(device), torch.cuda.stream(compute):
+            check(lib.sps_filter_scans_batch(lane_engine.handle, net.handle, map_hash.handle, _ptr(src), ld, h_off, batch,
+                                             _ptr(d_poses), float(eps), self.voxel_size, _ptr(rows), _ptr(row_offsets),
+                                             _ptr(n_rows), _ptr(counts), _ptr(scores), _ptr(metric_counts),
+                                             _ptr(metric_sums), _ptr(kept), _ptr(kept_offsets), _ptr(scratch), nbytes,
+                                             _stream(device)), "sps_filter_scans_batch")
+            out = FilteredScans(scores[:n], kept[:n], kept_offsets[:batch + 1], counts[:batch], metric_counts[:batch],
+                                metric_sums[:batch])
+            if on_device:
+                kept_end = grow("h_kept_end", (1,), torch.int32, True)
+                kept_end.copy_(kept_offsets[batch:batch + 1], non_blocking=True)
+            else:                                       # every result to pinned host memory, K not known yet
+                dev, out = out, FilteredScans(*(grow("h_" + name, (max(t.shape[0], 1),) + t.shape[1:], t.dtype, True)
+                                                [:t.shape[0]] for name, t in zip(FilteredScans._fields, out)))
+                for dst, t in zip(out, dev):
+                    dst.copy_(t, non_blocking=True)
+                kept_end = out.kept_offsets[batch:batch + 1]
+            done = torch.cuda.Event()
+            done.record(compute)
+        p["busy"][slot] = done
+        return _PendingFilter(done, out, lane_engine, kept_end)
 
     def _lane_forward(self, p, slot, lane_engine, net, src, d_out, compute):
         """One forward on a lane's stream (current), eagerly or as a CUDA-graph replay.  Every size that only exists on
