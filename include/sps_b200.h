@@ -309,6 +309,23 @@ int sps_filter_scans_batch(sps_ctx* ctx, const sps_net* net, const sps_map* map,
                            float* d_kept, int32_t* d_kept_offsets,
                            void* d_scratch, size_t scratch_bytes, void* stream);
 
+/* ---------------------------------------------------------------- sequence-sharded results ------- */
+/* Segments of a gathered buffer in sequence order (parallel.ShardedScans).  d_src fp32 [world][cap][width]: rank r's
+ * rows in block r (what a gather of per-rank [cap, width] buffers returns).  Segment s = rows h_seg_start[s] ..
+ * h_seg_start[s] + len_s of block h_seg_rank[s], where h_seg_rows[s] is the most rows it may hold (HOST arrays [n_seg])
+ * and len_s = d_seg_len[s] (DEVICE int32 [n_seg]) clamped to 0 .. h_seg_rows[s].  Outputs: d_out fp32
+ * [out_capacity, width] = segment 0's rows, then segment 1's, ...; d_out_offsets int32 [n_seg + 1] = where each segment
+ * starts in d_out (exclusive scan of the clamped lengths), d_out_offsets[n_seg] = the rows written.  One launch per
+ * 1 024 segments (each reads the previous one's total), float4 copies when width is a multiple of 4 and d_src and d_out
+ * are 16-byte aligned.  No host synchronisation.  SPS_ERR_BAD_ARG: world < 1, cap < 0, width < 1, n_seg < 0,
+ * out_capacity < 0, a null d_out_offsets, a null segment array with n_seg > 0, a null d_src or d_out when the segments
+ * can hold rows, a rank outside 0 .. world - 1, a negative start or row bound, h_seg_start[s] + h_seg_rows[s] > cap, a
+ * pointer that is not 4-byte aligned, world * cap * width beyond 2^59 elements, sum of h_seg_rows above 2^31 - 1;
+ * SPS_ERR_CAPACITY: out_capacity below the sum of h_seg_rows. */
+int sps_gather_segments(const float* d_src, int world, int64_t cap, int width, int n_seg, const int32_t* h_seg_rank,
+                        const int64_t* h_seg_start, const int64_t* h_seg_rows, const int32_t* d_seg_len, float* d_out,
+                        int64_t out_capacity, int32_t* d_out_offsets, void* stream);
+
 /* ---------------------------------------------------------------- ROS-path scan I/O (SURVEY 8f rank 3) --- */
 /* util.to_numpy (src/sps/datasets/util.py:146-153): the payload of a sensor_msgs/PointCloud2 -> fp32 [height*width,
  * nfields], every field cast to float32, fields in message order.  d_data: the message's `data` bytes on the device;

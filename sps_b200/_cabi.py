@@ -35,7 +35,7 @@ SYMBOLS = [
     "sps_ballmap_bytes", "sps_ballmap_build", "sps_ballmap_destroy", "sps_ball_query_scratch_bytes", "sps_submap_ball_query",
     "sps_radius_batch_scratch_bytes", "sps_radius_batch", "sps_predict_radius_batch",
     "sps_prune_batch_scratch_bytes", "sps_prune_batch", "sps_infer_prune_batch",
-    "sps_filter_scans_batch_scratch_bytes", "sps_filter_scans_batch",
+    "sps_filter_scans_batch_scratch_bytes", "sps_filter_scans_batch", "sps_gather_segments",
 ]
 
 
@@ -148,6 +148,7 @@ def load() -> C.CDLL:
         "sps_filter_scans_batch_scratch_bytes": (sz, [i64, i32]),
         "sps_filter_scans_batch": (i32, [vp, vp, vp, vp, i64, vp, i32, vp, f32, f32, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                           vp, sz, vp]),
+        "sps_gather_segments": (i32, [vp, i32, i64, i32, i32, vp, vp, vp, vp, vp, i64, vp, vp]),
         "sps_profile_enable": (i32, [vp, i32]),
         "sps_profile_read": (i32, [vp, vp, vp, i32, C.POINTER(i32)]),
         "sps_ctx_pair_count": (i32, [vp, i32, i32, C.POINTER(i64), vp]),

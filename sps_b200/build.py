@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsps_b200.so")
 STAMP = os.path.join(HERE, ".libsps_b200.stamp")
-SOURCES = ["api.cu", "maps.cu", "ballquery.cu", "rosio.cu", "conv_simt.cu", "conv_umma.cu", "net.cu"]
+SOURCES = ["api.cu", "maps.cu", "ballquery.cu", "rosio.cu", "shard.cu", "conv_simt.cu", "conv_umma.cu", "net.cu"]
 HEADERS = ["common.cuh", "ctx.h", "scan.cuh", "partials.cuh", "rosio.cuh", "umma_common.cuh", "profile.h",
            os.path.join("..", "..", "include", "sps_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

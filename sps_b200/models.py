@@ -152,10 +152,14 @@ class _Pending:
 
 
 class _PendingRadius:
-    """Handle of an in-flight ``SPSModel.predict_radius_async`` call."""
+    """Handle of an in-flight ``SPSModel.predict_radius_async`` call.  ``device_out`` (scan scores, counts, sums),
+    ``device_n_rows`` and ``row_capacity`` are the call's device results, its true row count and the rows its lane
+    held; they are valid on the lane's ``stream`` after the call and until the lane's next call."""
 
-    def __init__(self, event, out, engine, n_rows, retry):
+    def __init__(self, event, out, engine, n_rows, retry, device_out=None, device_n_rows=None, row_capacity=0,
+                 stream=None):
         self._event, self._out, self._engine, self._n_rows, self._retry = event, out, engine, n_rows, retry
+        self.device_out, self.device_n_rows, self.row_capacity, self.stream = device_out, device_n_rows, row_capacity, stream
 
     def result(self, check: bool = True):
         """Wait for the call and return ``(scan_scores, counts, sums)``.  ``check`` (default) also reads the engine's
@@ -183,11 +187,14 @@ class FilteredScans(NamedTuple):
 
 
 class _PendingFilter(_Pending):
-    """Handle of an in-flight ``SPSModel.filter_scans_async`` call."""
+    """Handle of an in-flight ``SPSModel.filter_scans_async`` call.  ``device_out`` is the call's :class:`FilteredScans`
+    on the device, ``kept`` with all ``sum n_b`` rows of the lane's buffer (the first ``kept_offsets[B]`` are the
+    published ones); it is valid on the lane's ``stream`` after the call and until the lane's next call."""
 
-    def __init__(self, event, out, engine, kept_end):
+    def __init__(self, event, out, engine, kept_end, device_out=None, stream=None):
         super().__init__(event, out, engine)
         self._kept_end = kept_end     # pinned host int32 [1]: K, once the call is done
+        self.device_out, self.stream = device_out, stream
 
     def result(self, check: bool = True) -> FilteredScans:
         """Wait for the call and return its :class:`FilteredScans` (``check``: as ``_Pending.result``)."""
@@ -410,7 +417,7 @@ class SPSModel(nn.Module):
                                                _ptr(rows), cap, _ptr(row_offsets), _ptr(n_rows), _ptr(scratch), nbytes,
                                                self.voxel_size, eps, _ptr(scores), _ptr(counts), _ptr(sums),
                                                _stream(device)), "sps_predict_radius_batch")
-            out = (scores[:n], counts[:batch], sums[:batch])
+            out = dev_out = (scores[:n], counts[:batch], sums[:batch])
             if not on_device:
                 h = (grow("h_scores", (max(n, 1),), torch.float32, True), grow("h_counts", (MAX_BATCH, 4), torch.int64, True),
                      grow("h_sums", (MAX_BATCH, 5), torch.float64, True))
@@ -425,7 +432,7 @@ class SPSModel(nn.Module):
 
         def retry(true_rows):
             return self._predict_radius(parts, offs, ld, submap, eps, true_rows)
-        return _PendingRadius(done, out, lane_engine, h_rows, retry)
+        return _PendingRadius(done, out, lane_engine, h_rows, retry, dev_out, n_rows, cap, compute)
 
     @staticmethod
     def _lane_scans(p, buf, grow, parts, n, ld, on_device, compute, device):
@@ -574,8 +581,8 @@ class SPSModel(nn.Module):
                                              _ptr(n_rows), _ptr(counts), _ptr(scores), _ptr(metric_counts),
                                              _ptr(metric_sums), _ptr(kept), _ptr(kept_offsets), _ptr(scratch), nbytes,
                                              _stream(device)), "sps_filter_scans_batch")
-            out = FilteredScans(scores[:n], kept[:n], kept_offsets[:batch + 1], counts[:batch], metric_counts[:batch],
-                                metric_sums[:batch])
+            out = dev_out = FilteredScans(scores[:n], kept[:n], kept_offsets[:batch + 1], counts[:batch],
+                                          metric_counts[:batch], metric_sums[:batch])
             if on_device:
                 kept_end = grow("h_kept_end", (1,), torch.int32, True)
                 kept_end.copy_(kept_offsets[batch:batch + 1], non_blocking=True)
@@ -588,7 +595,7 @@ class SPSModel(nn.Module):
             done = torch.cuda.Event()
             done.record(compute)
         p["busy"][slot] = done
-        return _PendingFilter(done, out, lane_engine, kept_end)
+        return _PendingFilter(done, out, lane_engine, kept_end, dev_out, compute)
 
     def _lane_forward(self, p, slot, lane_engine, net, src, d_out, compute):
         """One forward on a lane's stream (current), eagerly or as a CUDA-graph replay.  Every size that only exists on
