@@ -7,8 +7,9 @@
 // next tile's kernel-map slice, 54 % executing ~130 instructions per pipeline stage and only 8 % waiting for
 // a free stage.  Here
 //   * a dedicated LOADER warp builds the per-tile list of present offsets and stages the kernel-map
-//     slice (and the tile's own row numbers) up to 7 tiles ahead with 16-byte cp.async copies; a
-//     producer thread fetches the indices of its four rows with one 16-byte shared load;
+//     slice (and the tile's own row numbers) up to 8 tiles ahead with 16-byte cp.async copies, packed
+//     into a ring by the tiles' present offsets; a producer thread fetches the indices of its four
+//     rows with one 16-byte shared load;
 //   * the stage ring is 4 deep: the gathered rows are re-read from L1 by neighbouring output rows,
 //     and measured run time follows the L1 size the carve-out leaves (4 stages beat 2, 3 and 5-7;
 //     +40 KB of unused shared memory costs +25 % on the 32/48-channel layers).  A variant that
@@ -27,7 +28,7 @@
 namespace sps {
 
 // ring depth per accumulator width.  Round 1 ran ONE CTA per SM with a 4-deep ring (4 beat 2, 3 and 5-7).  Round 2: TWO
-// CTAs per SM, each with a 2-deep ring and one staged kernel-map slice (<= 113 KB of shared memory, <= 72 registers):
+// CTAs per SM, each with a 2-deep ring and the 42 KB index area (<= 113 KB of shared memory, <= 72 registers):
 // convolution family 1.79 -> 1.61 ms per forward (3-deep rings: 1.64) -- two independent gather streams fill the L1 data
 // pipe better than one deep ring, and the loader's bubble at a tile boundary hides behind the other CTA.
 constexpr int kV6CtasPerSm = 2;   // resident CTAs per SM for N <= 64 (the wide accumulators of the width sweep take a whole SM)
@@ -39,29 +40,35 @@ constexpr int kV6EpiWarp0 = kV6MmaWarp + 1;
 constexpr int kV6Threads = (kV6EpiWarp0 + 4) * 32;
 constexpr int kV6Entries = kMaxK + 1;                 // present offsets + the tile's own rows
 constexpr int kV6EntryBytes = kTileM * 4;
-// The index area (82 entries) holds as many tiles as fit: 1 for the 81-offset kernels, 8 for the 2x2x2 ones
-// (9 entries per tile).  Tiles of the small kernels are one or two stages long, so the number of tiles in flight
-// -- not the stage ring -- bounds their memory-level parallelism.
+// The index area (82 entries) is a ring: a tile takes nact + 1 consecutive entries (its present offsets, then its own
+// rows) from a running cursor, wrapping at the end, and the producers release tiles in order.  So the area holds as
+// many tiles as their PRESENT offsets allow, not K + 1 entries per tile: about three 81-offset tiles in shape-sorted
+// order (~22 offsets walked per tile; a tile with all 81 takes the whole area), eight of the 2x2x2 kernels (9 entries).
+// Without a second tile in flight the producers wait a full global round trip for the next slice at every tile
+// boundary; tiles of the small kernels are one or two stages long, so the number of tiles in flight -- not the stage
+// ring -- bounds their memory-level parallelism.
 constexpr int kV6MaxTilesAhead = 8;
-// ordered present-offset lists of the staged tiles: (K + 1) bytes each, rounded to 16 -> at most 224 bytes.  (Every
-// byte counts here: 167 936 bytes per CTA is the last size that still gets the 164 KB carve-out, i.e. 92 KB of L1.)
-constexpr int kV6KlistBytes = 256;
+// ordered present-offset lists of the staged tiles: one byte per ring entry (the kernel offset whose rows it holds)
+constexpr int kV6KlistBytes = (kV6Entries + 15) & ~15;
 
 template <int NPAD>
 struct V6Cfg {
   // SPS's own widths (N <= 64): 2 stages (above).  Wide accumulators of the width sweep (N = 128 / 256, 16 / 32 KB of
   // weights per stage): 4 / 3 stages -- a stage of such a layer keeps the tensor pipe busy for 256 / 512 cycles, the
-  // loader's bubble at a tile boundary is noise there.  Every width stages one tile's kernel-map slice.
+  // loader's bubble at a tile boundary is noise there.  Every width has the same index ring.
   static constexpr int S = NPAD == 256 ? 3 : NPAD == 128 ? 4 : 2;
   static constexpr int kBStage = NPAD * 128;
   static constexpr int kTmemCols = 2 * NPAD < 32 ? 32 : 2 * NPAD;
   static constexpr int kIdxEntries = kV6Entries;
   static constexpr int kShift = NPAD < 64 ? 64 : NPAD;
-  // A ring | B ring | row indices [kIdxEntries][128] | barriers | klists | nact [8] | shift | tmem slot
+  // A ring | B ring | row-index ring [kIdxEntries][128] | barriers | offset ring [kIdxEntries] | (start, nact) [8] |
+  // shift | tmem slot
   static constexpr size_t smem = (size_t)S * (kAStageBytes + kBStage) + (size_t)kIdxEntries * kV6EntryBytes +
-                                 8 * (2 * S + 2 * kV6MaxTilesAhead + 4) + kV6KlistBytes + 4 * kV6MaxTilesAhead +
+                                 8 * (2 * S + 2 * kV6MaxTilesAhead + 4) + kV6KlistBytes + 8 * kV6MaxTilesAhead +
                                  kShift * 4 + 16;
 };
+// two CTAs per SM: 228 KB of shared memory per SM, 1 KB of it reserved per CTA
+static_assert(kV6CtasPerSm * (V6Cfg<64>::smem + 1024) <= 228 * 1024, "two N <= 64 CTAs no longer fit on an SM");
 
 // 16-byte copy that writes zeros instead when `skip` is set (the ignore-src form: one predicate, no size select)
 template <bool kBypassL1>
@@ -112,8 +119,8 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
   uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(sidx) + Cfg::kIdxEntries * kV6EntryBytes);
   // bars: full[S], empty[S], idx_full[8], idx_empty[8], acc_full[2], acc_empty[2]
   uint8_t* klist = reinterpret_cast<uint8_t*>(bars + 2 * S + 2 * kV6MaxTilesAhead + 4);
-  int32_t* snact = reinterpret_cast<int32_t*>(klist + kV6KlistBytes);
-  float* sshift = reinterpret_cast<float*>(snact + kV6MaxTilesAhead);
+  int2* sslice = reinterpret_cast<int2*>(klist + kV6KlistBytes);   // per tile slot: first ring entry, present offsets
+  float* sshift = reinterpret_cast<float*>(sslice + kV6MaxTilesAhead);
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(sshift + Cfg::kShift);
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -171,10 +178,8 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
   const int st2 = in2_packed ? 0 : (gpk2 + 7) >> 3;     // stages of the fused 1x1 term
   const uint32_t* tmask = a.tile_mask;
   const int gstep = gridDim.x;
-  // tiles whose index slices fit in the staging area at once, and the bytes each takes
-  const int NP = min(kV6MaxTilesAhead, Cfg::kIdxEntries / (K + 1));
-  const uint32_t par_bytes = (uint32_t)(K + 1) * kV6EntryBytes;
-  const int kl_stride = (K + 1 + 15) & ~15;
+  // ring position of entry x of the tile whose entries start at `start`
+  auto ring = [](int start, int x) { const int q = start + x; return q >= Cfg::kIdxEntries ? q - Cfg::kIdxEntries : q; };
   auto tile_nact = [&](int tile) {
     return __popc(__ldg(tmask + 4 * tile)) + __popc(__ldg(tmask + 4 * tile + 1)) + __popc(__ldg(tmask + 4 * tile + 2));
   };
@@ -214,12 +219,11 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
 
     // ---- cursor over the stages of this CTA's tiles ----
     int tile = blockIdx.x, it_tile = 0;
-    int nact = 0, m = 0, nst = 0;                   // present offsets, current stage, stages of the tile
+    int start = 0, nact = 0, m = 0, nst = 0;        // first ring entry, present offsets, current stage, stages of the tile
     int ns_a = 0, ns_b = 0;                         // stages of the two channel segments of the tile
     bool stage_tma = false;                         // the weights of the stage about to be issued come through TMA
     int e = 0, sub = 0;                             // large Cin: offset entry and sub-stage
-    uint32_t sx = 0;                                // shared byte address of this thread's int4 in entry 0
-    const uint8_t* kl = klist;
+    const uint32_t sx = sidx_u + (uint32_t)r0 * 16u;   // shared byte address of this thread's int4 in ring entry 0
     // parameters of the stage about to be issued
     int idx[4] = {-1, -1, -1, -1};
     const char* base = in_b;
@@ -239,7 +243,8 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
           const int ee = m * EPS + e_off;
           const bool e_ok = ee < nact;
           const bool e_in2 = ee >= nact && ee < nact + n2;  // the slots after the last present offset: the 1x1 term
-          lds4(sx + (uint32_t)(e_ok ? ee : (e_in2 ? nact : 0)) * kV6EntryBytes);
+          const int pos = ring(start, e_ok ? ee : (e_in2 ? nact : 0));
+          lds4(sx + (uint32_t)pos * kV6EntryBytes);
           if (e_in2) {
             const int cg = (ee - nact) * GPCc + cg0;        // group of the in2 row this column carries
             base = in2_b + cg * 16; ld_b = in2_ld_b;
@@ -248,30 +253,32 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
           } else {
             base = in_b + cg0 * 16; ld_b = in_ld_b;
             okc = e_ok && cg0 < gpk; bok = e_ok;
-            wofs = (uint32_t)((int)kl[e_ok ? ee : 0] * GPCc + cg0) * 16u;
+            wofs = (uint32_t)((int)klist[pos] * GPCc + cg0) * 16u;
           }
           stage_tma = false;
         } else {
           // entry e = kernel offset klist[e], sub-stage `sub` of its SPE stages
-          if (sub == 0) lds4(sx + (uint32_t)e * kV6EntryBytes);
+          const int pos = ring(start, e);
+          if (sub == 0) lds4(sx + (uint32_t)pos * kV6EntryBytes);
           const int cg = cB + 8 * sub;
           base = in_b + cg * 16; ld_b = in_ld_b;
           okc = cg < gpk; bok = okc;
-          wofs = (uint32_t)((int)kl[e] * GP + cg) * 16u;
+          wofs = (uint32_t)((int)klist[pos] * GP + cg) * 16u;
           stage_tma = tma_b;
         }
       } else if (GPC2 && m < ns_a + ns_b) {
         const int ee = (m - ns_a) * EPS2 + e_off2;
         const bool e_ok = ee < nact;
-        lds4(sx + (uint32_t)(e_ok ? ee : 0) * kV6EntryBytes);
+        const int pos = ring(start, e_ok ? ee : 0);
+        lds4(sx + (uint32_t)pos * kV6EntryBytes);
         base = in_b + (gpk + cg02) * 16; ld_b = in_ld_b;
         okc = e_ok; bok = e_ok;
-        wofs = (uint32_t)(K * GP + (int)kl[e_ok ? ee : 0] * GPC2c + cg02) * 16u;
+        wofs = (uint32_t)(K * GP + (int)klist[pos] * GPC2c + cg02) * 16u;
         stage_tma = false;
       } else {
         // the fused 1x1 term on the tile's own rows (entry nact)
         const int cg = cB + 8 * (m - ns_a - ns_b);
-        lds4(sx + (uint32_t)nact * kV6EntryBytes);
+        lds4(sx + (uint32_t)ring(start, nact) * kV6EntryBytes);
         base = in2_b + cg * 16; ld_b = in2_ld_b;
         okc = cg < gpk2; bok = okc;
         wofs = (uint32_t)(K * (GP + GPC2) + cg) * 16u;
@@ -282,17 +289,16 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
     auto open_tile = [&]() -> bool {
       for (;;) {
         if (tile >= ntiles) return false;
-        const int par = it_tile % NP;
-        mbar_wait(bar_idxf + 8 * par, (it_tile / NP) & 1);
-        nact = snact[par];
+        const int slot = it_tile % kV6MaxTilesAhead;
+        mbar_wait(bar_idxf + 8 * slot, (it_tile / kV6MaxTilesAhead) & 1);
+        const int2 sl = sslice[slot];
+        start = sl.x; nact = sl.y;
         ns_a = stages_a(nact); ns_b = stages_b(nact);
         nst = ns_a + ns_b + st2;
-        sx = sidx_u + (uint32_t)par * par_bytes + (uint32_t)r0 * 16u;
-        kl = klist + par * kl_stride;
         m = 0; e = 0; sub = 0;
         if (nst > 0) { fetch(); return true; }
         __syncwarp();
-        if (lane == 0) mbar_arrive(bar_idxe + 8 * par);
+        if (lane == 0) mbar_arrive(bar_idxe + 8 * slot);
         tile += gstep; ++it_tile;
       }
     };
@@ -307,7 +313,7 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
         return true;
       }
       __syncwarp();                                   // every lane holds its indices in registers by now
-      if (lane == 0) mbar_arrive(bar_idxe + 8 * (it_tile % NP));
+      if (lane == 0) mbar_arrive(bar_idxe + 8 * (it_tile % kV6MaxTilesAhead));
       tile += gstep; ++it_tile;
       return open_tile();
     };
@@ -344,8 +350,9 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
     }
     cp_async_wait<0>();
   } else if (warp == kV6LoaderWarp) {
-    // =========================== LOADER (one warp, one tile ahead) ===========================
+    // =========================== LOADER (one warp, up to kV6MaxTilesAhead tiles ahead) ===========================
     int it = 0;
+    int head = 0, used = 0, it_free = 0;   // next free ring entry, entries held by tiles in flight, oldest tile in flight
     const bool map_vec = ((reinterpret_cast<uintptr_t>(a.map) & 15) == 0) && ((a.map_ld & 3) == 0);
     // the tile mask is the head of every tile's dependency chain: keep the NEXT tile's words in flight
     uint32_t mw[3] = {0u, 0u, 0u};
@@ -354,42 +361,50 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
       for (int w = 0; w < 3; ++w) mw[w] = __ldg(tmask + 4 * blockIdx.x + w);
     }
     for (int tile = blockIdx.x; tile < ntiles; tile += gstep, ++it) {
-      const int par = it % NP;
+      const int slot = it % kV6MaxTilesAhead;
       const uint32_t cur[3] = {mw[0], mw[1], mw[2]};
       if (tile + gstep < ntiles) {
 #pragma unroll
         for (int w = 0; w < 3; ++w) mw[w] = __ldg(tmask + 4 * (tile + gstep) + w);
       }
-      mbar_wait(bar_idxe + 8 * par, ((it / NP) & 1) ^ 1);     // producers are done with this buffer
-      uint8_t* klp = klist + par * kl_stride;
-      int nact = 0;
+      const int nact = __popc(cur[0]) + __popc(cur[1]) + __popc(cur[2]);
+      // wait until the tile's nact + 1 entries and its slot are free; the producers release tiles in order
+      while (it - it_free == kV6MaxTilesAhead || used + nact + 1 > Cfg::kIdxEntries) {
+        const int fs = it_free % kV6MaxTilesAhead;
+        mbar_wait(bar_idxe + 8 * fs, (it_free / kV6MaxTilesAhead) & 1);
+        used -= sslice[fs].y + 1;
+        ++it_free;
+      }
+      const int start = head;
+      head = ring(start, nact + 1);
+      used += nact + 1;
+      int n = 0;
 #pragma unroll
       for (int w = 0; w < 3; ++w) {
         const uint32_t bits = cur[w];
-        if ((bits >> lane) & 1u) klp[nact + __popc(bits & ((1u << lane) - 1u))] = (uint8_t)(32 * w + lane);
-        nact += __popc(bits);
+        if ((bits >> lane) & 1u) klist[ring(start, n + __popc(bits & ((1u << lane) - 1u)))] = (uint8_t)(32 * w + lane);
+        n += __popc(bits);
       }
-      if (lane == 0) snact[par] = nact;
+      if (lane == 0) sslice[slot] = make_int2(start, nact);
       __syncwarp();
       // entries are 128 row indices in tile order; lane owns rows 4 lane .. 4 lane + 3 (one 16-byte chunk per entry)
-      const uint32_t dst = sidx_u + (uint32_t)par * par_bytes + (uint32_t)lane * 16u;
+      const uint32_t dst0 = sidx_u + (uint32_t)lane * 16u;
+      auto dst = [&](int e) { return dst0 + (uint32_t)ring(start, e) * kV6EntryBytes; };
       if (a.tile_slices) {
         // the level's pass already gathered this tile's slice (entries 0..nact, the last one = own rows)
         const char* src = reinterpret_cast<const char*>(a.tile_slices + (int64_t)tile * (SPS_TILE_SLICE_ENTRIES * kTileM)) + lane * 16;
         for (int e = 0; e <= nact; ++e)
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + (uint32_t)e * kV6EntryBytes),
-                       "l"(src + (size_t)e * kV6EntryBytes)
+          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst(e)), "l"(src + (size_t)e * kV6EntryBytes)
                        : "memory");
       } else if (!a.perm && map_vec && !(p.flags & SPS_CONV_MAP_PARENT) && tile * kTileM + kTileM <= n_out) {
         // physical row order, full tile: the slice of map[k] is contiguous -> one 16-byte copy per lane and entry
         const int row0 = tile * kTileM + 4 * lane;
-        asm volatile("st.shared.v4.s32 [%0], {%1, %2, %3, %4};" ::"r"(dst + (uint32_t)nact * kV6EntryBytes), "r"(row0),
+        asm volatile("st.shared.v4.s32 [%0], {%1, %2, %3, %4};" ::"r"(dst(nact)), "r"(row0),
                      "r"(row0 + 1), "r"(row0 + 2), "r"(row0 + 3)
                      : "memory");
         const int32_t* src = a.map + row0;
         for (int e = 0; e < nact; ++e)
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst + (uint32_t)e * kV6EntryBytes),
-                       "l"(src + (int64_t)klp[e] * a.map_ld)
+          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst(e)), "l"(src + (int64_t)klist[ring(start, e)] * a.map_ld)
                        : "memory");
       } else {
         const int32_t* src[4];
@@ -403,13 +418,13 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
           const int row = rok[i] ? (a.perm ? __ldg(a.perm + prow) : prow) : 0;
           src[i] = a.map + row;
           pw[i] = (from_parent && rok[i]) ? __ldg(a.map + row) : -1;
-          asm volatile("st.shared.s32 [%0], %1;" ::"r"(dst + (uint32_t)nact * kV6EntryBytes + 4u * i), "r"(rok[i] ? row : -1) : "memory");
+          asm volatile("st.shared.s32 [%0], %1;" ::"r"(dst(nact) + 4u * i), "r"(rok[i] ? row : -1) : "memory");
         }
         for (int e = 0; e < nact; ++e) {
-          const int64_t koff = (int64_t)klp[e] * a.map_ld;
-          const uint32_t d = dst + (uint32_t)e * kV6EntryBytes;
+          const int k = klist[ring(start, e)];
+          const int64_t koff = (int64_t)k * a.map_ld;
+          const uint32_t d = dst(e);
           if (from_parent) {
-            const int k = klp[e];
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
               const int val = (pw[i] >= 0 && (pw[i] & 7) == k) ? (pw[i] >> 3) : -1;
@@ -424,9 +439,9 @@ __global__ void __launch_bounds__(kV6Threads, NPAD <= 64 ? kV6CtasPerSm : 1) k_c
           }
         }
       }
-      cp_async_arrive(bar_idxf + 8 * par);
+      cp_async_arrive(bar_idxf + 8 * slot);
       __syncwarp();
-      if (lane == 0) mbar_arrive(bar_idxf + 8 * par);         // orders the plain shared stores of the whole warp
+      if (lane == 0) mbar_arrive(bar_idxf + 8 * slot);        // orders the plain shared stores of the whole warp
     }
     cp_async_wait<0>();
   } else if (warp == kV6MmaWarp) {
